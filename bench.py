@@ -1,10 +1,14 @@
 #!/usr/bin/env python
-"""bench.py -- headline benchmark of the B200 audio->mesh hot path (contract in the task prompt / DESIGN.md).
+"""bench.py -- headline benchmark of the B200 audio->mesh hot path (DESIGN.md).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
                     [--workload faceformer|faceformer_train|audio2mesh|voca|voca_audio]   (configs[2] | [3] | [1] | [0]-shaped |
                                                                               raw audio windows -> MFCC -> VOCA)
     (configs[4], the long-sequence sweep: tools/sweep_long.py)
+
+--dump-outputs DIR writes the vertices the timed path returned in its last timed step to DIR/vertices.npy (float32,
+[n, 5023, 3]): a fixed, seeded sample of DUMP_MESHES meshes of the output, or all of them when it has fewer.  Inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.
 
 Workload (BASELINE.json configs[2], the largest single-GPU inference configuration): FaceFormer inference,
 random-init wav2vec2-base encoder + 1-layer biased causal decoder, batch 32 x 5 s synthetic 16 kHz audio at 30 fps,
@@ -100,6 +104,18 @@ class ClockSampler:
 
 
 _SD_CACHE = {}
+DUMP_MESHES = 512          # 512 x 5023 x 3 float32 = 31 MB
+
+
+def sample_meshes(out):
+    """--dump-outputs: the same DUMP_MESHES meshes of a [..., 5023, 3] output on every run (seeded choice over the
+    flattened leading dimensions, kept in order), as a float32 numpy array."""
+    import numpy as np
+    import torch
+    meshes = out.reshape(-1, 5023, 3)
+    n = meshes.shape[0]
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_MESHES), replace=False))
+    return meshes[torch.from_numpy(idx).to(meshes.device)].float().cpu().numpy()
 
 
 def deglitch(prof):
@@ -518,6 +534,7 @@ def run_ours(args, ctx):
         dev_s = sum(s.elapsed_time(e) for s, e in ev) * 1e-3
         n_par = {"faceformer": 1, "voca": 64}.get(args.workload, B)     # samples of the LAST TIMED step kept for the parity check
         timed_out = out[:n_par].detach().cpu() if rank == 0 else None
+        dump = sample_meshes(out) if rank == 0 and args.dump_outputs else None
         # ------------------------------ end-to-end timing (host buffers) ----------------------------
         # every step: H2D of the step's inputs from pinned memory, forward, D2H of the step's result into pinned
         # memory.  Copies run on a side stream so that step i's D2H overlaps step i+1's compute (double-buffered).
@@ -707,6 +724,10 @@ def run_ours(args, ctx):
         "cpu_baseline": cpu_baseline,
         "parity": infer_parity(args, timed_out, h_in),
     }
+    if dump is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "vertices.npy"), dump)
     return line
 
 
@@ -1026,7 +1047,7 @@ def run_sweep(args, ctx):
     m = m.to(dev).eval().set_precision("bf16")
     pk = peaks()
     rows = []
-    steps = max(2, min(args.steps, 3))
+    steps = args.steps
     for L_s, B_total in ((10.0, 128), (30.0, 32), (60.0, 8)):
         n = int(16000 * L_s)
         T = n * 60 // 16000
@@ -1106,10 +1127,17 @@ def main():
     ap.add_argument("--wire", default=None, choices=["fp32", "bf16"], help="faceformer_train: gradient all-reduce wire format "
                                                                              "(default: bf16 for the bf16 step)")
     ap.add_argument("--buckets", type=int, default=7, help="faceformer_train: all-reduce buckets per step (14 = one per stage)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="inference workloads: write the last timed step's vertices (a fixed sample of at most "
+                         f"{DUMP_MESHES} meshes) to DIR/vertices.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     with_extras = args.workload is None and not args.no_extra and args.impl == "ours"
     if args.workload is None:
         args.workload = "faceformer"
+    if args.dump_outputs and (args.impl != "ours" or args.workload in ("faceformer_train", "audio2mesh_train", "sweep")):
+        ap.error("--dump-outputs applies to the inference workloads of --impl ours")
     defaults = {"faceformer": 32, "faceformer_train": 8, "voca": 16384, "voca_config0": 348, "voca_audio": 4096, "audio2mesh": 64,
                 "audio2mesh_train": 128, "song2face": 64, "sweep": 0}
     if args.fps is None:
@@ -1133,7 +1161,7 @@ def main():
             sub = argparse.Namespace(**vars(args))
             sub.workload, sub.batch, sub.fps = wl, batch, fps if fps is not None else 30
             sub.seconds = 5.0
-            sub.steps = min(args.steps, 10)
+            sub.dump_outputs = None                 # the dump is the headline workload's output
             try:
                 extras[key] = run_one(sub, ctx)
             except Exception as exc:  # noqa: BLE001  (an extra leg must never take the headline line down with it)

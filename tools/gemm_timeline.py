@@ -1,5 +1,5 @@
 import sys, os
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from a2f_b200 import ops, lib as L
 dev = torch.device("cuda:0")
