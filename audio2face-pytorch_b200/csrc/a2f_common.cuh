@@ -162,6 +162,41 @@ A2F_D float ld_as_float(const bf16* p) { return __bfloat162float(*p); }
 A2F_D void st_from_float(float* p, float v) { *p = v; }
 A2F_D void st_from_float(bf16* p, float v) { *p = __float2bfloat16_rn(v); }
 
+// ---- dropout RNG (the contract is written down in include/a2f.h, "Encoder dropout") -----------------------------
+// Philox4x32-10 (Salmon et al., SC'11; the Random123 constants): counter c[4], key k[2].
+A2F_D uint4 philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        if (r) { k.x += 0x9E3779B9u; k.y += 0xBB67AE85u; }
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
+        c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+    }
+    return c;
+}
+
+// keep threshold: an element survives iff its 16-bit uniform is >= round(p * 65536)
+A2F_HD uint32_t dropout_threshold(float p) {
+    const float t = rintf(p * 65536.f);
+    return t <= 0.f ? 0u : (t >= 65536.f ? 65536u : (uint32_t)t);
+}
+
+// keep bits of the eight elements e = 8g .. 8g+7 of one site (bit i = element 8g+i); seed / offset as read from
+// a2f_dropout_args.seed_offset_dev.  Half-word i of the Philox output word i/2 (low half first) decides element 8g+i.
+A2F_D uint32_t dropout_keep8(unsigned long long seed, uint32_t offset, uint32_t site, unsigned long long g,
+                             uint32_t threshold) {
+    const uint4 r = philox4x32_10(make_uint4((uint32_t)g, (uint32_t)(g >> 32), site, offset),
+                                  make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+    const uint32_t w[4] = {r.x, r.y, r.z, r.w};
+    uint32_t bits = 0;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        const uint32_t u = (w[i >> 1] >> ((i & 1) * 16)) & 0xFFFFu;
+        bits |= (u >= threshold ? 1u : 0u) << i;
+    }
+    return bits;
+}
+
 A2F_D uint32_t pack_bf16x2(float lo, float hi) {
     __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
     return *reinterpret_cast<uint32_t*>(&v);

@@ -12,10 +12,47 @@
 
 namespace a2f {
 
+// ------------------------------------------------------------------------------------------------ dropout of P
+// Training with encoder dropout: O = (P o Z / (1 - p)) V with the LSE of the UNDROPPED softmax (HF modeling_wav2vec2.py
+// attention dropout).  Z follows the RNG contract of include/a2f.h over the logical tensor [B, H, T, Tp], Tp = ceil(T/8)*8:
+// keys 8k .. 8k+7 of query row t of (b, h) are ONE Philox call, g = ((b*H + h)*T + t)*Tp/8 + k, so the forward and both
+// backward passes regenerate the same bits from (seed, offset, site) whatever their tiling.  so == nullptr = off.
+struct AttnDrop {
+    const unsigned long long* so;     // {seed, offset} in device memory
+    uint32_t site, threshold;
+    float scale;                      // 1 / (1 - p)
+};
+struct AttnDropRt {                   // what a thread reads once at kernel start
+    unsigned long long seed;
+    uint32_t offset;
+};
+A2F_D AttnDropRt attn_drop_load(const AttnDrop& d) { return AttnDropRt{d.so[0], (uint32_t)d.so[1]}; }
+A2F_D uint32_t attn_keep8(const AttnDrop& d, const AttnDropRt& r, int bh, int T, int t, int ktile) {
+    const unsigned long long g = ((unsigned long long)bh * T + t) * (unsigned long long)((T + 7) >> 3) + ktile;
+    return dropout_keep8(r.seed, r.offset, d.site, g, d.threshold);
+}
+// Z of an m16n8k16 accumulator tile whose rows are queries (row_base + lane/4, +8) and whose n-tile nt holds keys
+// 8*(ktile0 + nt) + (lane&3)*2 + {0,1}: z[0] / z[1] = keep bits of the two rows' 8-key groups.  Each pair of n-tiles needs
+// 32 distinct Philox calls per warp, one per lane (call = row lane/4 bits 2-4, row half bit 1, n-tile parity bit 0),
+// computed at the even n-tile into `held` and handed out by shuffles.
+A2F_D void mma_rows_keep(const AttnDrop& d, const AttnDropRt& r, int bh, int T, int row_base, int ktile0, int nt, int lane,
+                         uint32_t& held, uint32_t* z) {
+    if ((nt & 1) == 0)
+        held = attn_keep8(d, r, bh, T, row_base + (lane >> 2) + 8 * ((lane >> 1) & 1), ktile0 + nt + (lane & 1));
+    z[0] = __shfl_sync(0xffffffffu, held, (lane & ~3) | (nt & 1));
+    z[1] = __shfl_sync(0xffffffffu, held, (lane & ~3) | 2 | (nt & 1));
+}
+A2F_D void mask_pair(uint32_t z, int lane, float& a, float& b) {
+    const int c = (lane & 3) * 2;
+    if (!((z >> c) & 1u)) a = 0.f;
+    if (!((z >> (c + 1)) & 1u)) b = 0.f;
+}
+
 // ------------------------------------------------------------------------------------------------ fp32 SIMT
 // qkv: [B,T,3*H*64] fp32.  One warp per (b,h,query).  Lane l scores keys j = j0+l; output dims (2l, 2l+1).
 __global__ void __launch_bounds__(256) mha_f32_kernel(const float* __restrict__ qkv, float* __restrict__ out,
-                                                      float* __restrict__ lse, int B, int T, int H, float scale) {
+                                                      float* __restrict__ lse, int B, int T, int H, float scale,
+                                                      AttnDrop drop) {
     const int warp_global = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     const int total = B * H * T;
@@ -32,6 +69,8 @@ __global__ void __launch_bounds__(256) mha_f32_kernel(const float* __restrict__ 
         const float4 f = *reinterpret_cast<const float4*>(qp + d);
         q[d] = f.x; q[d + 1] = f.y; q[d + 2] = f.z; q[d + 3] = f.w;
     }
+    const bool dropping = drop.so != nullptr;
+    const AttnDropRt dr = dropping ? attn_drop_load(drop) : AttnDropRt{0ull, 0u};
     float m = -INFINITY, l = 0.f, o0 = 0.f, o1 = 0.f;
     for (int j0 = 0; j0 < T; j0 += 32) {
         const int j = j0 + lane;
@@ -53,18 +92,20 @@ __global__ void __launch_bounds__(256) mha_f32_kernel(const float* __restrict__ 
         const float corr = __expf(m - m_new);      // first chunk: exp(-inf) = 0
         const float pj = (j < T) ? __expf(s - m_new) : 0.f;
         l = l * corr + warp_sum(pj);
+        float pd = pj;                                    // the dropped probability feeds O, the undropped one l / LSE
+        if (dropping && j < T && !((attn_keep8(drop, dr, b * H + h, T, t, j >> 3) >> (j & 7)) & 1u)) pd = 0.f;
         o0 *= corr;
         o1 *= corr;
         const int nj = min(32, T - j0);
         for (int jj = 0; jj < nj; ++jj) {
-            const float pv = __shfl_sync(0xffffffffu, pj, jj);
+            const float pv = __shfl_sync(0xffffffffu, pd, jj);
             const float2 vv = *reinterpret_cast<const float2*>(base + (long long)(j0 + jj) * ld + 2 * H * 64 + h * 64 + 2 * lane);
             o0 = fmaf(pv, vv.x, o0);
             o1 = fmaf(pv, vv.y, o1);
         }
         m = m_new;
     }
-    const float inv = 1.f / l;
+    const float inv = (dropping ? drop.scale : 1.f) / l;
     float* op = out + ((long long)b * T + t) * (H * 64) + h * 64 + 2 * lane;
     *reinterpret_cast<float2*>(op) = make_float2(o0 * inv, o1 * inv);
     if (lse != nullptr && lane == 0) lse[((long long)b * H + h) * T + t] = m + logf(l);
@@ -100,9 +141,10 @@ A2F_D void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory
 template <int N> A2F_D void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 // grid: (ceil(T/64), H, B); 128 threads.
+template <bool DROP>
 __global__ void __launch_bounds__(128) mha_bf16_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out,
                                                        float* __restrict__ lse, float* __restrict__ out32, int T, int H,
-                                                       float scale_log2) {
+                                                       float scale_log2, AttnDrop drop) {
     pdl_sync();   // PDL: wait for the previous kernel's results, let the next kernel's prologue start
     __shared__ __align__(16) bf16 sQ[FA_BM * FA_LD];
     __shared__ __align__(16) bf16 sK[2][FA_BN * FA_LD];
@@ -140,6 +182,8 @@ __global__ void __launch_bounds__(128) mha_bf16_kernel(const bf16* __restrict__ 
 #pragma unroll
         for (int j = 0; j < 4; ++j) o[i][j] = 0.f;
     float m_run[2] = {-INFINITY, -INFINITY}, l_run[2] = {0.f, 0.f};
+    AttnDropRt dr{0ull, 0u};
+    if (DROP) dr = attn_drop_load(drop);
 
     for (int it = 0; it < ntiles; ++it) {
         const int cur = it & 1;
@@ -210,14 +254,21 @@ __global__ void __launch_bounds__(128) mha_bf16_kernel(const bf16* __restrict__ 
         }
         float rs[2] = {0.f, 0.f};
         uint32_t pf[4][4];                 // P as A fragments: 4 k-steps of 16 keys
+        uint32_t zheld = 0;
 #pragma unroll
         for (int nt = 0; nt < 8; ++nt) {
-            const float p0 = exp2f(fmaf(s[nt][0], scale_log2, -msc[0]));
-            const float p1 = exp2f(fmaf(s[nt][1], scale_log2, -msc[0]));
-            const float p2 = exp2f(fmaf(s[nt][2], scale_log2, -msc[1]));
-            const float p3 = exp2f(fmaf(s[nt][3], scale_log2, -msc[1]));
+            float p0 = exp2f(fmaf(s[nt][0], scale_log2, -msc[0]));
+            float p1 = exp2f(fmaf(s[nt][1], scale_log2, -msc[0]));
+            float p2 = exp2f(fmaf(s[nt][2], scale_log2, -msc[1]));
+            float p3 = exp2f(fmaf(s[nt][3], scale_log2, -msc[1]));
             rs[0] += p0 + p1;
             rs[1] += p2 + p3;
+            if (DROP) {
+                uint32_t z[2];
+                mma_rows_keep(drop, dr, b * H + h, T, q0 + warp * 16, key0 / 8, nt, lane, zheld, z);
+                mask_pair(z[0], lane, p0, p1);
+                mask_pair(z[1], lane, p2, p3);
+            }
             const int ks = nt >> 1, hi = nt & 1;
             pf[ks][hi * 2 + 0] = pack_bf16x2(p0, p1);
             pf[ks][hi * 2 + 1] = pack_bf16x2(p2, p3);
@@ -253,7 +304,8 @@ __global__ void __launch_bounds__(128) mha_bf16_kernel(const bf16* __restrict__ 
         l_run[r] += __shfl_xor_sync(0xffffffffu, l_run[r], 2);
     }
     const int row0 = q0 + warp * 16 + (lane >> 2);
-    const float inv0 = 1.f / l_run[0], inv1 = 1.f / l_run[1];
+    const float osc = DROP ? drop.scale : 1.f;
+    const float inv0 = osc / l_run[0], inv1 = osc / l_run[1];
     if (lse != nullptr && (lane & 3) == 0) {
         // natural-log LSE of the scaled scores: m*scale + ln(l)
         float* lp = lse + ((long long)b * H + h) * T;
@@ -301,10 +353,10 @@ template <int NKT, int NQB> struct FsCfg {
 };
 
 // grid: (ceil(T/(80*NQB)), H, B); 160 threads; T <= NKT*16.
-template <int NKT, int NQB>
+template <int NKT, int NQB, bool DROP>
 __global__ void __launch_bounds__(32 * FS_NW, 3) mha_short_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out,
                                                                    float* __restrict__ lse, float* __restrict__ out32, int T,
-                                                                   int H, float scale_log2) {
+                                                                   int H, float scale_log2, AttnDrop drop) {
     constexpr int KEYS = NKT * 16;
     extern __shared__ __align__(16) uint8_t fs_smem[];
     bf16* sQ = reinterpret_cast<bf16*>(fs_smem);
@@ -382,14 +434,23 @@ __global__ void __launch_bounds__(32 * FS_NW, 3) mha_short_kernel(const bf16* __
             mx[r] = fmaxf(mx[r], __shfl_xor_sync(0xffffffffu, mx[r], 2));
         }
         const float msc0 = mx[0] * scale_log2, msc1 = mx[1] * scale_log2;
+        AttnDropRt dr{0ull, 0u};
+        if (DROP) dr = attn_drop_load(drop);
+        uint32_t zheld = 0;
 #pragma unroll
         for (int nt = 0; nt < 2 * NKT; ++nt) {
-            const float p0 = exp2f(fmaf(s[nt][0], scale_log2, -msc0));
-            const float p1 = exp2f(fmaf(s[nt][1], scale_log2, -msc0));
-            const float p2 = exp2f(fmaf(s[nt][2], scale_log2, -msc1));
-            const float p3 = exp2f(fmaf(s[nt][3], scale_log2, -msc1));
+            float p0 = exp2f(fmaf(s[nt][0], scale_log2, -msc0));
+            float p1 = exp2f(fmaf(s[nt][1], scale_log2, -msc0));
+            float p2 = exp2f(fmaf(s[nt][2], scale_log2, -msc1));
+            float p3 = exp2f(fmaf(s[nt][3], scale_log2, -msc1));
             rs[0] += p0 + p1;
             rs[1] += p2 + p3;
+            if (DROP) {
+                uint32_t z[2];
+                mma_rows_keep(drop, dr, b * H + h, T, q0 + qrow, 0, nt, lane, zheld, z);
+                mask_pair(z[0], lane, p0, p1);
+                mask_pair(z[1], lane, p2, p3);
+            }
             const int ks = nt >> 1, hi = nt & 1;
             pf[ks][hi * 2 + 0] = pack_bf16x2(p0, p1);
             pf[ks][hi * 2 + 1] = pack_bf16x2(p2, p3);
@@ -424,7 +485,8 @@ __global__ void __launch_bounds__(32 * FS_NW, 3) mha_short_kernel(const bf16* __
         rs[r] += __shfl_xor_sync(0xffffffffu, rs[r], 2);
     }
     const int row0 = q0 + qrow + (lane >> 2);
-    const float inv0 = 1.f / rs[0], inv1 = 1.f / rs[1];
+    const float osc = DROP ? drop.scale : 1.f;
+    const float inv0 = osc / rs[0], inv1 = osc / rs[1];
     if (lse != nullptr && (lane & 3) == 0) {
         float* lp = lse + ((long long)b * H + h) * T;
         if (row0 < T) lp[row0] = mx[0] * scale_log2 * 0.69314718055994531f + logf(rs[0]);
@@ -453,28 +515,30 @@ __global__ void __launch_bounds__(32 * FS_NW, 3) mha_short_kernel(const bf16* __
   }   // qb
 }
 
-template <int NKT, int NQB>
+template <int NKT, int NQB, bool DROP>
 static int launch_mha_short_q(const bf16* qkv, bf16* out, float* lse, float* out32, int B, int T, int H, float scale_log2,
-                              cudaStream_t s) {
-    auto kern = mha_short_kernel<NKT, NQB>;
+                              const AttnDrop& drop, cudaStream_t s) {
+    auto kern = mha_short_kernel<NKT, NQB, DROP>;
     static bool attr_done = false;
     if (!attr_done) {
         A2F_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FsCfg<NKT, NQB>::SMEM_BYTES));
         attr_done = true;
     }
     const dim3 grid((T + NQB * FS_BM - 1) / (NQB * FS_BM), H, B);
-    A2F_CHECK_CUDA(launch_pdl(kern, grid, dim3(32 * FS_NW), FsCfg<NKT, NQB>::SMEM_BYTES, s, qkv, out, lse, out32, T, H, scale_log2));
+    A2F_CHECK_CUDA(launch_pdl(kern, grid, dim3(32 * FS_NW), FsCfg<NKT, NQB>::SMEM_BYTES, s, qkv, out, lse, out32, T, H, scale_log2,
+                              drop));
     return A2F_OK;
 }
 
 static int g_mha_short_nqb = 0;   // debug: 0 = automatic (2 query blocks per CTA when T > 80), 1 = one block per CTA (round 1)
 void set_mha_short_nqb(int v) { g_mha_short_nqb = v; }
 
-template <int NKT>
+template <int NKT, bool DROP>
 static int launch_mha_short(const bf16* qkv, bf16* out, float* lse, float* out32, int B, int T, int H, float scale_log2,
-                            cudaStream_t s) {
-    if (T > FS_BM && g_mha_short_nqb != 1) return launch_mha_short_q<NKT, 2>(qkv, out, lse, out32, B, T, H, scale_log2, s);
-    return launch_mha_short_q<NKT, 1>(qkv, out, lse, out32, B, T, H, scale_log2, s);
+                            const AttnDrop& drop, cudaStream_t s) {
+    if (T > FS_BM && g_mha_short_nqb != 1)
+        return launch_mha_short_q<NKT, 2, DROP>(qkv, out, lse, out32, B, T, H, scale_log2, drop, s);
+    return launch_mha_short_q<NKT, 1, DROP>(qkv, out, lse, out32, B, T, H, scale_log2, drop, s);
 }
 
 
@@ -499,7 +563,8 @@ __global__ void __launch_bounds__(256) mha_delta_kernel(const TO* __restrict__ o
 // fp32 parity path: one warp per (b,h,query); lanes own keys; dK / dV through fp32 atomics (dqkv must be zeroed).
 __global__ void __launch_bounds__(128) mha_bwd_f32_kernel(const float* __restrict__ qkv, const float* __restrict__ dout,
                                                           const float* __restrict__ lse, const float* __restrict__ delta,
-                                                          float* __restrict__ dqkv, int B, int T, int H, float scale) {
+                                                          float* __restrict__ dqkv, int B, int T, int H, float scale,
+                                                          AttnDrop drop) {
     __shared__ float qs[4][64], dos[4][64];
     const int wl = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int wg = blockIdx.x * 4 + wl;
@@ -514,6 +579,8 @@ __global__ void __launch_bounds__(128) mha_bwd_f32_kernel(const float* __restric
     dos[wl][lane + 32] = dout[((long long)b * T + t) * (H * 64) + h * 64 + lane + 32];
     __syncwarp();
     const float L = lse[((long long)b * H + h) * T + t], dl = delta[((long long)b * H + h) * T + t];
+    const bool dropping = drop.so != nullptr;
+    const AttnDropRt dr = dropping ? attn_drop_load(drop) : AttnDropRt{0ull, 0u};
     float dq[64];
 #pragma unroll
     for (int d = 0; d < 64; ++d) dq[d] = 0.f;
@@ -531,6 +598,13 @@ __global__ void __launch_bounds__(128) mha_bwd_f32_kernel(const float* __restric
             dp = fmaf(dos[wl][d + 2], vf.z, dp); dp = fmaf(dos[wl][d + 3], vf.w, dp);
         }
         const float p = __expf(s * scale - L);
+        // dropout: O = (P o Z/(1-p)) V, so dV sees the dropped P and dP = (dO V^T) o Z/(1-p); delta = rowsum(dO o O) holds
+        float pv = p;
+        if (dropping) {
+            const float z = ((attn_keep8(drop, dr, b * H + h, T, t, j >> 3) >> (j & 7)) & 1u) ? drop.scale : 0.f;
+            pv = p * z;
+            dp *= z;
+        }
         const float ds = p * (dp - dl) * scale;
         float* dkp = dbase + (long long)j * ld + H * 64 + h * 64;
         float* dvp = dbase + (long long)j * ld + 2 * H * 64 + h * 64;
@@ -538,7 +612,7 @@ __global__ void __launch_bounds__(128) mha_bwd_f32_kernel(const float* __restric
         for (int d = 0; d < 64; ++d) {
             dq[d] = fmaf(ds, kp[d], dq[d]);
             atomicAdd(dkp + d, ds * qs[wl][d]);
-            atomicAdd(dvp + d, p * dos[wl][d]);
+            atomicAdd(dvp + d, pv * dos[wl][d]);
         }
     }
     float* dqp = dbase + (long long)t * ld + h * 64;
@@ -552,9 +626,10 @@ __global__ void __launch_bounds__(128) mha_bwd_f32_kernel(const float* __restric
 constexpr int FAB_TILE = FA_BM * FA_LD;     // bf16 elements of one 64 x 64 (padded) tile
 
 // bf16 tensor-core backward, query-major pass: dQ = (P o (dO V^T - delta)) K * scale.   grid (ceil(T/64), H, B), 128 thr.
+template <bool DROP>
 __global__ void __launch_bounds__(128) mha_bwd_dq_kernel(const bf16* __restrict__ qkv, const bf16* __restrict__ dout,
                                                          const float* __restrict__ lse, const float* __restrict__ delta,
-                                                         bf16* __restrict__ dqkv, int T, int H, float scale) {
+                                                         bf16* __restrict__ dqkv, int T, int H, float scale, AttnDrop drop) {
     extern __shared__ __align__(16) bf16 fab_smem[];
     bf16* sQ = fab_smem;
     bf16* sdO = sQ + FAB_TILE;
@@ -591,6 +666,8 @@ __global__ void __launch_bounds__(128) mha_bwd_dq_kernel(const bf16* __restrict_
     lse2[1] = r0 + 8 < T ? lp[r0 + 8] * 1.4426950408889634f : 0.f;
     dl[0] = r0 < T ? dp_[r0] : 0.f;
     dl[1] = r0 + 8 < T ? dp_[r0 + 8] : 0.f;
+    AttnDropRt dr{0ull, 0u};
+    if (DROP) dr = attn_drop_load(drop);
     uint32_t qf[4][4], dof[4][4];
     float dq[8][4];
 #pragma unroll
@@ -642,16 +719,25 @@ __global__ void __launch_bounds__(128) mha_bwd_dq_kernel(const bf16* __restrict_
         }
         const int key0 = it * FA_BN;
         uint32_t dsf[4][4];
+        uint32_t zheld = 0;
 #pragma unroll
         for (int nt = 0; nt < 8; ++nt) {
             const int kc = key0 + nt * 8 + (lane & 3) * 2;
+            float zs[4] = {1.f, 1.f, 1.f, 1.f};
+            if (DROP) {                    // dP = (dO V^T) o Z/(1-p)
+                uint32_t z[2];
+                mma_rows_keep(drop, dr, b * H + h, T, q0 + warp * 16, key0 / 8, nt, lane, zheld, z);
+                const int c = (lane & 3) * 2;
+#pragma unroll
+                for (int e = 0; e < 4; ++e) zs[e] = ((z[e >> 1] >> (c + (e & 1))) & 1u) ? drop.scale : 0.f;
+            }
             float d4[4];
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
                 const int rr = e >> 1;
                 const bool ok = (kc + (e & 1)) < T;
                 const float p = ok ? exp2f(fmaf(s[nt][e], scale_log2, -lse2[rr])) : 0.f;
-                d4[e] = p * (dp[nt][e] - dl[rr]) * scale;
+                d4[e] = p * (dp[nt][e] * zs[e] - dl[rr]) * scale;
             }
             const int ks = nt >> 1, hi = nt & 1;
             dsf[ks][hi * 2 + 0] = pack_bf16x2(d4[0], d4[1]);
@@ -681,9 +767,10 @@ __global__ void __launch_bounds__(128) mha_bwd_dq_kernel(const bf16* __restrict_
 }
 
 // key-major pass: dV = P^T dO, dK = (P o (dO V^T - delta))^T Q * scale.   grid (ceil(T/64), H, B), 128 threads.
+template <bool DROP>
 __global__ void __launch_bounds__(128) mha_bwd_dkv_kernel(const bf16* __restrict__ qkv, const bf16* __restrict__ dout,
                                                           const float* __restrict__ lse, const float* __restrict__ delta,
-                                                          bf16* __restrict__ dqkv, int T, int H, float scale) {
+                                                          bf16* __restrict__ dqkv, int T, int H, float scale, AttnDrop drop) {
     extern __shared__ __align__(16) bf16 fab_smem[];
     bf16* sK = fab_smem;
     bf16* sV = sK + FAB_TILE;
@@ -724,6 +811,8 @@ __global__ void __launch_bounds__(128) mha_bwd_dkv_kernel(const bf16* __restrict
     load_stats(0, 0);
     cp_async_commit();
     const float scale_log2 = scale * 1.4426950408889634f;
+    AttnDropRt dr{0ull, 0u};
+    if (DROP) dr = attn_drop_load(drop);
     uint32_t kf[4][4], vf[4][4];
     float dk[8][4], dv[8][4];
 #pragma unroll
@@ -777,17 +866,33 @@ __global__ void __launch_bounds__(128) mha_bwd_dkv_kernel(const bf16* __restrict
         }
         const int qbase = it * FA_BM;
         uint32_t pf[4][4], dsf[4][4];
+        uint32_t zbits_dkv = 0;
 #pragma unroll
         for (int nt = 0; nt < 8; ++nt) {
             const int qc = nt * 8 + (lane & 3) * 2;         // query column within the tile
+            float zs[4] = {1.f, 1.f, 1.f, 1.f};
+            if (DROP) {
+                // rows here are KEYS (k0 + warp*16 + lane/4, +8), columns queries: per pair of n-tiles one Philox call per
+                // lane, call (query pair slot, query parity, key group, n-tile parity) = lane bits (0-1, 2, 3, 4)
+                if ((nt & 1) == 0) {
+                    const int q = qbase + (nt + (lane >> 4)) * 8 + (lane & 3) * 2 + ((lane >> 2) & 1);
+                    zbits_dkv = attn_keep8(drop, dr, b * H + h, T, q, (k0 + warp * 16) / 8 + ((lane >> 3) & 1));
+                }
+#pragma unroll
+                for (int e = 0; e < 4; ++e) {
+                    const int src = (lane & 3) | ((e & 1) << 2) | ((e >> 1) << 3) | ((nt & 1) << 4);
+                    const uint32_t zb = __shfl_sync(0xffffffffu, zbits_dkv, src);
+                    zs[e] = ((zb >> (lane >> 2)) & 1u) ? drop.scale : 0.f;
+                }
+            }
             float p4[4], d4[4];
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
                 const int qq = qc + (e & 1);
                 const bool ok = (qbase + qq) < T;
                 const float p = ok ? exp2f(fmaf(st[nt][e], scale_log2, -sL[cur * 64 + qq])) : 0.f;
-                p4[e] = p;
-                d4[e] = p * (dpt[nt][e] - sD[cur * 64 + qq]) * scale;
+                p4[e] = p * zs[e];                                 // dV = (P o Z/(1-p))^T dO
+                d4[e] = p * (dpt[nt][e] * zs[e] - sD[cur * 64 + qq]) * scale;
             }
             const int ks = nt >> 1, hi = nt & 1;
             pf[ks][hi * 2 + 0] = pack_bf16x2(p4[0], p4[1]);
@@ -844,6 +949,17 @@ void set_mha_tc_min_t(int v) { g_mha_tc_min_t = v; }
 
 using namespace a2f;
 
+// attention dropout of a2f_dropout_args (NULL / p == 0 / NULL pointer = off)
+static int attn_drop_from(const a2f_dropout_args* a, AttnDrop* d, bool* on) {
+    *d = AttnDrop{nullptr, 0u, 0u, 1.f};
+    *on = false;
+    if (a == nullptr || a->seed_offset_dev == nullptr || a->p == 0.f) return A2F_OK;
+    if (!(a->p > 0.f && a->p < 1.f)) return set_error(A2F_EINVAL, "attention dropout: p must lie in [0, 1)");
+    *d = AttnDrop{static_cast<const unsigned long long*>(a->seed_offset_dev), a->site, dropout_threshold(a->p), 1.f / (1.f - a->p)};
+    *on = true;
+    return A2F_OK;
+}
+
 extern "C" int a2f_mha_fwd(const void* qkv, void* out, int dtype, int B, int T, int H, int D, float scale,
                            void* stream) {
     return a2f_mha_fwd_train(qkv, out, nullptr, nullptr, dtype, B, T, H, D, scale, stream);
@@ -863,21 +979,34 @@ extern "C" int a2f_mha_bwd(const void* qkv, const void* out, const void* dout, c
 extern "C" int a2f_mha_bwd_train(const void* qkv, const void* out, const float* out_f32, const void* dout, const float* lse,
                                  void* dqkv, int dtype, int B, int T, int H, int D, float scale, void* workspace,
                                  size_t workspace_bytes, void* stream) {
+    return a2f_mha_bwd_train_dropout(qkv, out, out_f32, dout, lse, dqkv, dtype, B, T, H, D, scale, nullptr, workspace,
+                                     workspace_bytes, stream);
+}
+
+extern "C" int a2f_mha_bwd_train_dropout(const void* qkv, const void* out, const float* out_f32, const void* dout,
+                                         const float* lse, void* dqkv, int dtype, int B, int T, int H, int D, float scale,
+                                         const a2f_dropout_args* dropout, void* workspace, size_t workspace_bytes,
+                                         void* stream) {
     int rc = require_sm100();
     if (rc != A2F_OK) return rc;
     A2F_REQUIRE(qkv && out && dout && lse && dqkv && workspace && B > 0 && T > 0 && H > 0, "a2f_mha_bwd: bad arguments");
     A2F_REQUIRE(D == 64, "a2f_mha_bwd: head_dim must be 64");
     A2F_REQUIRE(workspace_bytes >= (size_t)B * H * T * sizeof(float), "a2f_mha_bwd: workspace too small (B*H*T floats)");
+    AttnDrop drop;
+    bool dropping;
+    rc = attn_drop_from(dropout, &drop, &dropping);
+    if (rc != A2F_OK) return rc;
     cudaStream_t s = as_stream(stream);
     float* delta = static_cast<float*>(workspace);
     const long long warps = (long long)B * T * H;
     const int dgrid = (int)((warps * 32 + 255) / 256);
+    // delta = rowsum(dO o O) with the DROPPED output O (what the forward returned): still rowsum(dP o P) of the softmax
     if (dtype == A2F_F32) {
         mha_delta_kernel<float, float><<<dgrid, 256, 0, s>>>((const float*)out, (const float*)dout, delta, B, T, H);
         A2F_CHECK_LAUNCH("mha_delta_kernel");
         A2F_CHECK_CUDA(cudaMemsetAsync(dqkv, 0, (size_t)B * T * 3 * H * 64 * sizeof(float), s));
         mha_bwd_f32_kernel<<<(int)((warps + 3) / 4), 128, 0, s>>>((const float*)qkv, (const float*)dout, lse, delta,
-                                                                  (float*)dqkv, B, T, H, scale);
+                                                                  (float*)dqkv, B, T, H, scale, drop);
         A2F_CHECK_LAUNCH("mha_bwd_f32_kernel");
         count_launch(2);
     } else if (dtype == A2F_BF16) {
@@ -889,14 +1018,18 @@ extern "C" int a2f_mha_bwd_train(const void* qkv, const void* out, const float* 
         const size_t smem = (size_t)6 * FAB_TILE * sizeof(bf16) + 256 * sizeof(float);
         static bool attr_done = false;
         if (!attr_done) {
-            A2F_CHECK_CUDA(cudaFuncSetAttribute(mha_bwd_dq_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            A2F_CHECK_CUDA(cudaFuncSetAttribute(mha_bwd_dkv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            A2F_CHECK_CUDA(cudaFuncSetAttribute(mha_bwd_dq_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            A2F_CHECK_CUDA(cudaFuncSetAttribute(mha_bwd_dkv_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            A2F_CHECK_CUDA(cudaFuncSetAttribute(mha_bwd_dq_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            A2F_CHECK_CUDA(cudaFuncSetAttribute(mha_bwd_dkv_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             attr_done = true;
         }
         const dim3 grid((T + 63) / 64, H, B);
-        mha_bwd_dq_kernel<<<grid, 128, smem, s>>>((const bf16*)qkv, (const bf16*)dout, lse, delta, (bf16*)dqkv, T, H, scale);
+        auto dq = dropping ? mha_bwd_dq_kernel<true> : mha_bwd_dq_kernel<false>;
+        auto dkv = dropping ? mha_bwd_dkv_kernel<true> : mha_bwd_dkv_kernel<false>;
+        dq<<<grid, 128, smem, s>>>((const bf16*)qkv, (const bf16*)dout, lse, delta, (bf16*)dqkv, T, H, scale, drop);
         A2F_CHECK_LAUNCH("mha_bwd_dq_kernel");
-        mha_bwd_dkv_kernel<<<grid, 128, smem, s>>>((const bf16*)qkv, (const bf16*)dout, lse, delta, (bf16*)dqkv, T, H, scale);
+        dkv<<<grid, 128, smem, s>>>((const bf16*)qkv, (const bf16*)dout, lse, delta, (bf16*)dqkv, T, H, scale, drop);
         A2F_CHECK_LAUNCH("mha_bwd_dkv_kernel");
         count_launch(3);
     } else {
@@ -907,22 +1040,31 @@ extern "C" int a2f_mha_bwd_train(const void* qkv, const void* out, const float* 
 
 extern "C" int a2f_mha_fwd_train(const void* qkv, void* out, float* lse, float* out_f32, int dtype, int B, int T, int H,
                                  int D, float scale, void* stream) {
+    return a2f_mha_fwd_train_dropout(qkv, out, lse, out_f32, dtype, B, T, H, D, scale, nullptr, stream);
+}
+
+extern "C" int a2f_mha_fwd_train_dropout(const void* qkv, void* out, float* lse, float* out_f32, int dtype, int B, int T,
+                                         int H, int D, float scale, const a2f_dropout_args* dropout, void* stream) {
     int rc = require_sm100();
     if (rc != A2F_OK) return rc;
     A2F_REQUIRE(qkv && out && B > 0 && T > 0 && H > 0, "a2f_mha_fwd: bad arguments");
     A2F_REQUIRE(D == 64, "a2f_mha_fwd: head_dim must be 64");
+    AttnDrop drop;
+    bool dropping;
+    rc = attn_drop_from(dropout, &drop, &dropping);
+    if (rc != A2F_OK) return rc;
     cudaStream_t s = as_stream(stream);
     if (dtype == A2F_F32) {
         const long long warps = (long long)B * H * T;
         const int grid = (int)((warps * 32 + 255) / 256);
-        mha_f32_kernel<<<grid, 256, 0, s>>>(static_cast<const float*>(qkv), static_cast<float*>(out), lse, B, T, H, scale);
+        mha_f32_kernel<<<grid, 256, 0, s>>>(static_cast<const float*>(qkv), static_cast<float*>(out), lse, B, T, H, scale, drop);
         A2F_CHECK_LAUNCH("mha_f32_kernel");
     } else if (dtype == A2F_BF16) {
         A2F_REQUIRE(reinterpret_cast<uintptr_t>(qkv) % 16 == 0, "a2f_mha_fwd: qkv must be 16-byte aligned");
         // inference forward (no log-sum-exp / fp32 side output): the tcgen05 kernel of attention_tc.cu for sequences
         // long enough to fill its 128x128 tiles; the mma.sync kernel below for short ones and for training
         const int impl = mha_impl();
-        if (lse == nullptr && out_f32 == nullptr && reinterpret_cast<uintptr_t>(out) % 16 == 0 &&
+        if (!dropping && lse == nullptr && out_f32 == nullptr && reinterpret_cast<uintptr_t>(out) % 16 == 0 &&
             (impl == 2 || (impl == 0 && T >= mha_tc_min_t()))) {
             rc = mha_tc_fwd(qkv, out, B, T, H, scale, s);
             if (rc != A2F_OK) return rc;
@@ -932,15 +1074,22 @@ extern "C" int a2f_mha_fwd_train(const void* qkv, void* out, float* lse, float* 
         if (impl != 1 && T <= 160) {
             // short clips: single-pass kernel with every key of a (batch, head) resident in shared memory
             const float sl2 = scale * 1.4426950408889634f;
-            rc = T <= 80 ? launch_mha_short<5>(static_cast<const bf16*>(qkv), static_cast<bf16*>(out), lse, out_f32, B, T, H, sl2, s)
-                         : launch_mha_short<10>(static_cast<const bf16*>(qkv), static_cast<bf16*>(out), lse, out_f32, B, T, H, sl2, s);
+            const bf16* q = static_cast<const bf16*>(qkv);
+            bf16* o = static_cast<bf16*>(out);
+            if (dropping)
+                rc = T <= 80 ? launch_mha_short<5, true>(q, o, lse, out_f32, B, T, H, sl2, drop, s)
+                             : launch_mha_short<10, true>(q, o, lse, out_f32, B, T, H, sl2, drop, s);
+            else
+                rc = T <= 80 ? launch_mha_short<5, false>(q, o, lse, out_f32, B, T, H, sl2, drop, s)
+                             : launch_mha_short<10, false>(q, o, lse, out_f32, B, T, H, sl2, drop, s);
             if (rc != A2F_OK) return rc;
             count_launch();
             return A2F_OK;
         }
         const dim3 grid((T + FA_BM - 1) / FA_BM, H, B);
-        A2F_CHECK_CUDA(launch_pdl(mha_bf16_kernel, dim3(grid), dim3(128), 0, s, static_cast<const bf16*>(qkv), static_cast<bf16*>(out), lse, out_f32, T, H,
-                                              scale * 1.4426950408889634f));
+        auto kern = dropping ? mha_bf16_kernel<true> : mha_bf16_kernel<false>;
+        A2F_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(128), 0, s, static_cast<const bf16*>(qkv), static_cast<bf16*>(out), lse,
+                                  out_f32, T, H, scale * 1.4426950408889634f, drop));
         A2F_CHECK_LAUNCH("mha_bf16_kernel");
     } else {
         return set_error(A2F_EINVAL, "a2f_mha_fwd: bad dtype");

@@ -78,6 +78,16 @@ class EncoderBlockArgs(C.Structure):
     ]
 
 
+class DropoutArgs(C.Structure):
+    """a2f_dropout_args (include/a2f.h): drop probability, site id, device pointer to {seed, offset} (int64 x 2)."""
+    _fields_ = [("p", c_float), ("site", C.c_uint), ("seed_offset_dev", c_void_p)]
+
+
+# site ids of the encoder dropout RNG contract (include/a2f.h): 8 * layer + kind, and the two pre-layer sites
+DROP_ATTN_PROB, DROP_ATTN_OUT, DROP_FFN_ACT, DROP_FFN_OUT = 0, 1, 2, 3
+DROP_FEAT_PROJ, DROP_ENC_IN = 96, 97
+
+
 class DecoderWeights(C.Structure):
     _names = [
         "sa_in_w", "sa_in_b", "sa_out_w", "sa_out_b", "ca_in_w", "ca_in_b", "ca_out_w", "ca_out_b",
@@ -132,6 +142,10 @@ _SIGNATURES = {
     "a2f_mha_fwd_train": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p]),
     "a2f_mha_bwd_train": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
                                   c_float, c_void_p, c_size_t, c_void_p]),
+    "a2f_mha_fwd_train_dropout": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_float,
+                                          C.POINTER(DropoutArgs), c_void_p]),
+    "a2f_mha_bwd_train_dropout": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
+                                          c_int, c_float, C.POINTER(DropoutArgs), c_void_p, c_size_t, c_void_p]),
     "a2f_decoder_workspace_bytes": (c_size_t, [c_int, c_int]),
     "a2f_decoder_rollout_ca": (c_int, [C.POINTER(DecoderWeights), c_void_p, c_void_p, c_int, c_int, c_void_p, c_int,
                                     c_int, c_void_p, c_size_t, c_void_p]),
@@ -175,6 +189,8 @@ _SIGNATURES = {
     "a2f_transpose_cast": (c_int, [c_void_p, c_ll, c_ll, c_int, c_int, c_void_p, c_int, c_ll, c_void_p]),
     "a2f_add_strided3": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_ll, c_ll, c_ll, c_ll, c_ll, c_ll, c_void_p]),
     "a2f_colsum": (c_int, [c_void_p, c_int, c_ll, c_ll, c_int, c_void_p, c_void_p]),
+    "a2f_dropout_mask": (c_int, [C.POINTER(DropoutArgs), c_ll, c_void_p, c_void_p]),
+    "a2f_dropout_apply": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_ll, C.POINTER(DropoutArgs), c_void_p]),
     "a2f_spec_mask_fwd": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_ll, c_int, c_void_p]),
     "a2f_spec_mask_bwd": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_ll, c_int, c_void_p]),
     "a2f_layernorm_bwd": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_float, c_void_p, c_int, c_void_p,

@@ -569,6 +569,18 @@ class Faceformer(_A2FModule):
         # reference's host-side numpy draws (spec_augment.py).  None = follow self.training like the reference does;
         # True / False force it.
         self.spec_augment = None
+        # training forward only (train() mode, training.forward_train): the wav2vec2 encoder's train-mode dropout and
+        # LayerDrop (HF modeling_wav2vec2.py).  False (default) = eval arithmetic.  True applies, with the probabilities of
+        # dropout_p, dropout after the feature projection ("feat_proj"), after encoder.layer_norm and on both residual
+        # branches of every layer ("hidden"), on the attention probabilities ("attention"), on the FFN activation
+        # ("activation"), and skips whole layers ("layerdrop").  The decoder / PPE dropout is not applied.  A no-grad
+        # forward is the inference path and stays eval arithmetic.  The defaults are the 960h checkpoint config the
+        # reference loads; "feat_proj" = 0.1 is from SURVEY.md A.4, which gives it from memory (not verifiable offline).
+        self.encoder_dropout = False
+        self.dropout_p = {"hidden": 0.1, "attention": 0.1, "activation": 0.1, "feat_proj": 0.1, "layerdrop": 0.1}
+        # Philox key of the dropout masks and seed of the LayerDrop draws (include/a2f.h); None = drawn from torch's default
+        # generator at first use; FaceformerTrainer gives every replica rank 0's seed.
+        self.dropout_seed = None
         # bf16 inference: run the encoder's 24 post-LayerNorms inside the GEMM epilogues (a2f_gemm_ln); False = the separate
         # layernorm_kernel launches (A/B switch for profiles/)
         self.fuse_layernorm = True

@@ -725,6 +725,36 @@ def colsum3(x: torch.Tensor, outs) -> None:
                                  outs[2].data_ptr(), _stream()), "a2f_colsum3")
 
 
+def _dropout_args(p: float, site: int, seed_offset: Optional[torch.Tensor]) -> "L.DropoutArgs":
+    if seed_offset is not None:
+        _dev(seed_offset)
+        if seed_offset.dtype != torch.int64 or seed_offset.numel() != 2 or not seed_offset.is_contiguous():
+            raise L.A2FError("dropout: seed_offset is a contiguous int64 device tensor {seed, offset}")
+    return L.DropoutArgs(float(p), int(site), L.ptr(seed_offset))
+
+
+def dropout_mask(p: float, site: int, seed_offset: torch.Tensor, shape) -> torch.Tensor:
+    """Keep mask (uint8, 1 = kept) of one dropout site over its logical tensor `shape` (RNG contract, include/a2f.h)."""
+    mask = torch.empty(tuple(shape), dtype=torch.uint8, device=seed_offset.device)
+    L.check(L.load().a2f_dropout_mask(C.byref(_dropout_args(p, site, seed_offset)), mask.numel(), mask.data_ptr(),
+                                      _stream()), "a2f_dropout_mask")
+    return mask
+
+
+def dropout_apply(x: torch.Tensor, p: float, site: int, seed_offset: torch.Tensor, resid: Optional[torch.Tensor] = None,
+                  out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """out = drop(x) [+ resid] (out may be x or resid); also the backward of the site when x is its gradient."""
+    _dev(x, resid, out)
+    if out is None:
+        out = torch.empty_like(x)
+    for t in (x, resid, out):
+        if t is not None and (t.dtype != x.dtype or not t.is_contiguous() or t.numel() != x.numel()):
+            raise L.A2FError("dropout_apply: x, resid and out are contiguous tensors of one dtype and size")
+    L.check(L.load().a2f_dropout_apply(x.data_ptr(), L.ptr(resid), out.data_ptr(), _dt(x), x.numel(),
+                                       C.byref(_dropout_args(p, site, seed_offset)), _stream()), "a2f_dropout_apply")
+    return out
+
+
 def spec_mask_fwd(h: torch.Tensor, mask_u8: torch.Tensor, embed: torch.Tensor) -> torch.Tensor:
     """h[mask] = embed, in place (ref:src/model/wav2vec.py:159-161).  h [rows, cols], mask_u8 uint8 [rows]."""
     _dev(h, mask_u8, embed)
@@ -871,23 +901,35 @@ def weight_norm_bwd(dwp, v, g, dv, dg):
                                          ws.data_ptr(), 256 * 8, _stream()), "a2f_weight_norm_bwd")
 
 
-def mha_lse(qkv, out, lse, B, T, H=12, D=64, scale=0.125, out_f32: Optional[torch.Tensor] = None):
-    """training forward: also the row log-sum-exp and (bf16 path, optional) the un-rounded fp32 output."""
+def mha_lse(qkv, out, lse, B, T, H=12, D=64, scale=0.125, out_f32: Optional[torch.Tensor] = None, dropout=None):
+    """training forward: also the row log-sum-exp and (bf16 path, optional) the un-rounded fp32 output.
+    dropout: None, or (p, site, seed_offset) -- attention-probability dropout (a2f_mha_fwd_train_dropout)."""
     _dev(qkv, out, lse, out_f32)
     if out_f32 is not None and (out_f32.dtype != torch.float32 or qkv.dtype != torch.bfloat16):
         raise L.A2FError("out_f32 is the fp32 side output of the bf16 attention kernel")
-    L.check(L.load().a2f_mha_fwd_train(qkv.data_ptr(), out.data_ptr(), lse.data_ptr(), L.ptr(out_f32), _dt(qkv), B, T, H, D,
-                                       scale, _stream()), "a2f_mha_fwd_train")
+    if dropout is None:
+        L.check(L.load().a2f_mha_fwd_train(qkv.data_ptr(), out.data_ptr(), lse.data_ptr(), L.ptr(out_f32), _dt(qkv), B, T, H,
+                                           D, scale, _stream()), "a2f_mha_fwd_train")
+        return out
+    L.check(L.load().a2f_mha_fwd_train_dropout(qkv.data_ptr(), out.data_ptr(), lse.data_ptr(), L.ptr(out_f32), _dt(qkv), B, T,
+                                               H, D, scale, C.byref(_dropout_args(*dropout)), _stream()),
+            "a2f_mha_fwd_train_dropout")
     return out
 
 
-def mha_bwd(qkv, out, dout, lse, B, T, H=12, D=64, scale=0.125, out_f32: Optional[torch.Tensor] = None):
+def mha_bwd(qkv, out, dout, lse, B, T, H=12, D=64, scale=0.125, out_f32: Optional[torch.Tensor] = None, dropout=None):
+    """dropout: the forward's (p, site, seed_offset), whose mask the backward regenerates."""
     _dev(qkv, out, dout, lse, out_f32)
     dqkv = torch.empty_like(qkv)
     ws = torch.empty(B * H * T, dtype=torch.float32, device=qkv.device)
-    L.check(L.load().a2f_mha_bwd_train(qkv.data_ptr(), out.data_ptr(), L.ptr(out_f32), dout.data_ptr(), lse.data_ptr(),
-                                       dqkv.data_ptr(), _dt(qkv), B, T, H, D, scale, ws.data_ptr(), ws.numel() * 4, _stream()),
-            "a2f_mha_bwd_train")
+    if dropout is None:
+        L.check(L.load().a2f_mha_bwd_train(qkv.data_ptr(), out.data_ptr(), L.ptr(out_f32), dout.data_ptr(), lse.data_ptr(),
+                                           dqkv.data_ptr(), _dt(qkv), B, T, H, D, scale, ws.data_ptr(), ws.numel() * 4,
+                                           _stream()), "a2f_mha_bwd_train")
+        return dqkv
+    L.check(L.load().a2f_mha_bwd_train_dropout(qkv.data_ptr(), out.data_ptr(), L.ptr(out_f32), dout.data_ptr(), lse.data_ptr(),
+                                               dqkv.data_ptr(), _dt(qkv), B, T, H, D, scale, C.byref(_dropout_args(*dropout)),
+                                               ws.data_ptr(), ws.numel() * 4, _stream()), "a2f_mha_bwd_train_dropout")
     return dqkv
 
 

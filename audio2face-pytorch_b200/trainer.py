@@ -181,7 +181,11 @@ class FlatBuffers:
 class FaceformerTrainer:
     """One process per GPU.  `step(audio, one_hot, template, gt)` = forward + FaceFormerLoss + backward + gradient
     all-reduce + Adam, in the units it is given; `training_step(batch)` applies the reference's x100 scaling first
-    (ref:src/model/lightning_model.py:145-148).  Eval-mode arithmetic (dropout / LayerDrop / SpecAugment off, DESIGN.md).
+    (ref:src/model/lightning_model.py:145-148).  Eval-mode arithmetic by default (dropout / LayerDrop / SpecAugment off,
+    DESIGN.md); `model.encoder_dropout = True` in train() mode turns on the wav2vec2 encoder's dropout and LayerDrop.
+    The rank is folded into the dropout key (replicas draw independent masks); LayerDrop draws from the seed alone
+    (every replica skips the same layers).  A layer skipped by LayerDrop gets no gradient, and like torch.optim.Adam
+    for `grad is None`, its parameters, moments and step count stay untouched that step.
 
     Batch semantics (extension; the reference is batch-1): loss = mean over the utterances of the per-utterance
     FaceFormerLoss; across ranks the gradient is the average of the per-rank gradients (DDP semantics)."""
@@ -210,6 +214,18 @@ class FaceformerTrainer:
         self.flat.bump_versions()
         self._ws = None
         self._step_dev = torch.zeros(1, dtype=torch.int32, device=self.flat.params.device)
+        if _world() > 1:
+            # one dropout seed for all replicas (rank 0's, drawn there if unset): LayerDrop must skip the same layers on
+            # every rank, and the rank is folded into the Philox key so that the dropout masks differ
+            seed = torch.tensor([-1 if model.dropout_seed is None else int(model.dropout_seed)], dtype=torch.int64,
+                                device=self.flat.params.device)
+            if dist.get_rank(group) == 0 and model.dropout_seed is None:
+                seed.fill_(int(torch.randint(0, 2 ** 62, (1,)).item()))
+            dist.broadcast(seed, src=dist.get_global_rank(group, 0) if group is not None else 0, group=group)
+            model.dropout_seed = int(seed.item())
+        training.set_dropout_rank(model, dist.get_rank() if _world() > 1 else 0)
+        self._skipped_stages = frozenset()      # stages of the layers LayerDrop skipped in the last forward
+        self._stage_steps = None                # per-stage Adam step counts once LayerDrop has skipped a stage
         self.fuse_loss = True          # bf16 path: vertex head + losses in one kernel (False = head, loss_fwd, loss_bwd, cast)
         self._dy = None
         self._ws_head = None
@@ -225,6 +241,7 @@ class FaceformerTrainer:
         one_hot = one_hot.reshape(B, -1).contiguous().float()
         tmpl = template.reshape(B, -1).contiguous().float()
         self.flat.zero_grads()
+        self._skipped_stages = frozenset()
         hook = (lambda st: self.flat.all_reduce_stage(st, self.group)) if (self.overlap and _world() > 1) else None
         T = audio.shape[1] * self.fps // 16000
         if self.fuse_loss and m.precision == "bf16" and T >= 2 and T % 2 == 0:
@@ -234,6 +251,7 @@ class FaceformerTrainer:
             # and take the unfused path below.)
             with torch.no_grad():
                 _, tape = training.forward_train(m, audio, one_hot, tmpl, self.fps, with_head=False)
+                self._note_skips(tape)
                 V3, M = m.vertice_dim, B * T
                 g = gt.reshape(M, V3)
                 if g.dtype != torch.float32 or not g.is_contiguous():
@@ -250,6 +268,7 @@ class FaceformerTrainer:
             return out3
         with torch.no_grad():
             out, tape = training.forward_train(m, audio, one_hot, tmpl, self.fps)
+            self._note_skips(tape)
             T, V3 = out.shape[1], m.vertice_dim
             Te = T - (T % 2)                                  # ref loss.py:12-15: an odd last frame is dropped
             if Te < 2:
@@ -273,10 +292,46 @@ class FaceformerTrainer:
             training.backward(m, tape, dpred, on_ready=hook)
         return out3
 
+    def _note_skips(self, tape) -> None:
+        from . import training
+        drop = tape.get("drop")
+        if drop and drop["skip"]:
+            self._skipped_stages = frozenset(training.grad_stage_of(f"audio_encoder.encoder.layers.{l}.") for l in drop["skip"])
+
+    def _adam_per_stage(self) -> None:
+        """Adam over the stages that received gradients, each run of consecutive stages with equal step counts in one
+        launch (eager only: the counts are host-side)."""
+        from . import ops
+        n = len(self.flat.stage_ranges)
+        if self._stage_steps is None:
+            self._stage_steps = [self.steps - 1] * n
+        g = self.flat.reduced_grads()
+        runs = []
+        for st in range(n):
+            if st in self._skipped_stages:
+                continue
+            self._stage_steps[st] += 1
+            if runs and runs[-1][1] == st - 1 and self._stage_steps[runs[-1][0]] == self._stage_steps[st]:
+                runs[-1][1] = st
+            else:
+                runs.append([st, st])
+        for s0, s1 in runs:
+            lo, hi = self.flat.stage_ranges[s0][0], self.flat.stage_ranges[s1][1]
+            if hi > lo:
+                ops.adam_step(self.flat.params[lo:hi], g[lo:hi], self.exp_avg[lo:hi], self.exp_avg_sq[lo:hi], self.lr,
+                              self.betas[0], self.betas[1], self.eps, self.weight_decay, self._stage_steps[s0],
+                              grad_scale=1.0 / _world())
+
     def optimizer_step(self) -> None:
         from . import ops
         self.flat.finish_all_reduce(self.group)
         self.steps += 1
+        if self._skipped_stages or self._stage_steps is not None:
+            # LayerDrop skipped a layer (now or earlier): per-parameter step counts differ, as in torch.optim.Adam
+            self._step_dev.add_(1)
+            self._adam_per_stage()
+            self.flat.bump_versions()
+            return
         # the step count lives on the device (incremented on the stream) so that the whole step can be replayed as a graph
         self._step_dev.add_(1)
         ops.adam_step(self.flat.params, self.flat.reduced_grads(), self.exp_avg, self.exp_avg_sq, self.lr, self.betas[0],
@@ -309,13 +364,20 @@ class GraphedTrainStep:
     all-reduce and the fused Adam update -- captured as ONE CUDA graph for fixed shapes.  A step is ~330 launches of mostly
     small kernels; replaying the graph takes the Python / ctypes launch path (15-25 us per launch on the host) off the
     critical path.  Call it like `step`: inputs are copied into the captured buffers; the returned loss tensors are the
-    captured outputs (overwritten by the next replay).  Requirements: eval-mode arithmetic (no host-side SpecAugment draw
-    inside the step) and shapes equal to the captured ones."""
+    captured outputs (overwritten by the next replay).  Requirements: no host-side draw inside the step (SpecAugment and
+    LayerDrop off; encoder dropout is fine, each replay draws fresh masks) and shapes equal to the captured ones."""
 
     def __init__(self, trainer: "FaceformerTrainer", audio, one_hot, template, gt, warmup: int = 2):
         from . import training
         if training.spec_augment_active(trainer.model):
             raise L.A2FError("GraphedTrainStep: SpecAugment draws its mask on the host every step; capture needs it off")
+        m = trainer.model
+        if training.encoder_dropout_active(m) and float({**training.DROPOUT_DEFAULTS, **(m.dropout_p or {})}["layerdrop"]) > 0:
+            raise L.A2FError("GraphedTrainStep: LayerDrop draws the skipped layers on the host every step; capture needs "
+                             "dropout_p['layerdrop'] = 0 (dropout alone is captured: its offset advances on the device)")
+        if trainer._stage_steps is not None:
+            raise L.A2FError("GraphedTrainStep: LayerDrop left per-stage Adam step counts; capture needs a trainer that never "
+                             "skipped a layer")
         self.trainer = trainer
         self.static_in = [audio.clone(), one_hot.clone(), template.clone(), gt.clone()]
         side = torch.cuda.Stream()

@@ -2,8 +2,10 @@
 backward pass (ref: torch.autograd over ref:src/model/faceformer.py:139-188 + HF Wav2Vec2Model inside Lightning's
 training_step, ref:src/model/lightning_model.py:150-161).
 
-Semantics: eval-mode arithmetic by default (dropout and LayerDrop are inactive -- stated in DESIGN.md; torch's
-device-side RNG makes bit-level parity of those ops meaningless).  SpecAugment, whose randomness is host-side numpy in
+Semantics: eval-mode arithmetic by default (dropout and LayerDrop are inactive -- stated in DESIGN.md).  With
+`model.encoder_dropout = True` a training forward in train() mode applies the wav2vec2 encoder's dropout sites and
+LayerDrop (see encoder_dropout_active); its masks follow the RNG contract of include/a2f.h, so oracle/philox.py can
+regenerate them exactly.  SpecAugment, whose randomness is host-side numpy in
 the reference, is available with `model.spec_augment = True` and reproduces the reference's masks draw for draw
 (spec_augment.py).  Every parameter of the reference receives a gradient; `audio_encoder.masked_spec_embed` only with
 SpecAugment on (same in the reference: unused otherwise, SURVEY.md App. B.2).  Parameter gradients are ACCUMULATED into `param.grad` (allocated as zeros when
@@ -30,6 +32,11 @@ V3PAD = 15072          # 15069 rounded up to a multiple of 8 (16-byte bf16 rows 
 
 
 _WARNED_DROPOUT = False
+
+# wav2vec2 encoder dropout (modules.Faceformer.dropout_p): the 960h checkpoint config the reference loads
+DROPOUT_DEFAULTS = {"hidden": 0.1, "attention": 0.1, "activation": 0.1, "feat_proj": 0.1, "layerdrop": 0.1}
+N_ENC_LAYERS = 12
+_RANK_MIX = 0x9E3779B97F4A7C15          # replicas' Philox keys: seed ^ (rank * _RANK_MIX) mod 2^64
 _GRAD_SINK = None      # set by collect_grads(): id(param) -> buffer the explicit backward accumulates into instead of .grad
 
 
@@ -78,6 +85,74 @@ class collect_grads:
     def grads(self):
         """One entry per parameter: its gradient, or None when the backward never wrote it / it does not require grad."""
         return tuple(self.bufs[id(p)] if (id(p) in self.touched and p.requires_grad) else None for p in self.params)
+
+
+def encoder_dropout_active(model) -> bool:
+    """Encoder dropout / LayerDrop run in a training forward when `model.encoder_dropout` is True and the module is in
+    train() mode.  A no-grad forward (Faceformer.forward under torch.no_grad) is the inference path and keeps eval
+    arithmetic either way."""
+    return bool(getattr(model, "encoder_dropout", False)) and model.training
+
+
+def _i64(v: int) -> int:
+    v &= (1 << 64) - 1
+    return v - (1 << 64) if v >= 1 << 63 else v
+
+
+def dropout_key(seed: int, rank: int = 0) -> int:
+    """64-bit Philox key of a replica: the seed itself on rank 0, so replicas draw independent masks."""
+    return (int(seed) ^ (int(rank) * _RANK_MIX)) & ((1 << 64) - 1)
+
+
+def _dropout_state(model, dev) -> torch.Tensor:
+    """The model's device int64 {key, offset}, plus the host generator of the LayerDrop draws (seeded with the seed alone,
+    so every replica skips the same layers without a collective).  Created at first use (seed drawn from torch's default
+    generator when model.dropout_seed is None); a new model.dropout_seed starts a new stream (offset 0, generator
+    reseeded), a new rank a new key, and a device move carries the offset over."""
+    if getattr(model, "dropout_seed", None) is None:
+        model.dropout_seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+    seed, rank = int(model.dropout_seed), getattr(model, "_dropout_rank", 0)
+    st, meta = getattr(model, "_drop_state", None), getattr(model, "_drop_meta", None)
+    if st is not None and meta == (seed, rank, dev):
+        return st
+    offset = 0
+    if st is not None and meta[0] == seed:
+        offset = int(st[1])                      # same stream on a new device or under a new rank
+    else:
+        model._layerdrop_gen = torch.Generator().manual_seed(seed)
+    st = torch.tensor([_i64(dropout_key(seed, rank)), offset], dtype=torch.int64, device=dev)
+    model._drop_state, model._drop_meta = st, (seed, rank, dev)
+    return st
+
+
+def set_dropout_rank(model, rank: int) -> None:
+    """Fold the data-parallel rank into the model's dropout key (FaceformerTrainer does this at construction)."""
+    model._dropout_rank = int(rank)
+
+
+def _draw_layerdrop(model, p: float) -> frozenset:
+    """Layers skipped by this forward: one host uniform per layer, like HF's `torch.rand([]) < layerdrop`."""
+    if p <= 0:
+        return frozenset()
+    u = torch.rand(N_ENC_LAYERS, generator=model._layerdrop_gen)
+    return frozenset(i for i in range(N_ENC_LAYERS) if float(u[i]) < p)
+
+
+def _dropout_plan(model, dev) -> Optional[Dict]:
+    """Snapshot (seed, offset) for this forward and its backward, advance the model's offset on the stream, draw
+    LayerDrop.  None when encoder dropout is off."""
+    if not encoder_dropout_active(model):
+        return None
+    p = dict(DROPOUT_DEFAULTS)
+    p.update(getattr(model, "dropout_p", None) or {})
+    for k, v in p.items():
+        if not 0.0 <= float(v) < 1.0:
+            raise L.A2FError(f"dropout_p[{k!r}] = {v} must lie in [0, 1)")
+    st = _dropout_state(model, dev)
+    so = st.clone()
+    st[1:].add_(1)
+    return {"so": so, "hidden": float(p["hidden"]), "activation": float(p["activation"]), "attention": float(p["attention"]),
+            "feat_proj": float(p["feat_proj"]), "skip": _draw_layerdrop(model, float(p["layerdrop"]))}
 
 
 def conv_lengths(n_samples: int) -> List[int]:
@@ -176,11 +251,16 @@ def forward_train(model, audio: torch.Tensor, one_hot: torch.Tensor, tmpl: torch
     global _WARNED_DROPOUT
     if model.training and not _WARNED_DROPOUT:
         # the reference's train() mode also enables dropout 0.1 (PPE, decoder layer, wav2vec2 hidden / activation / attention)
-        # and LayerDrop 0.1; this path applies SpecAugment only.  Said once, loudly, because a drop-in must not hide it.
+        # and LayerDrop 0.1.  Said once, loudly, because a drop-in must not hide what is missing.
         import warnings
-        warnings.warn("a2f_b200 Faceformer in train() mode: SpecAugment is applied like the reference's, but dropout (p=0.1) and "
-                      "LayerDrop are NOT -- the training kernels run eval-mode arithmetic for those ops (INTEGRATION.md 2c)",
-                      RuntimeWarning, stacklevel=3)
+        if encoder_dropout_active(model):
+            msg = ("a2f_b200 Faceformer in train() mode with encoder_dropout: SpecAugment and the wav2vec2 encoder's dropout "
+                   "and LayerDrop are applied, but the decoder / PPE dropout is NOT (INTEGRATION.md 2c)")
+        else:
+            msg = ("a2f_b200 Faceformer in train() mode: SpecAugment is applied like the reference's, but dropout (p=0.1) and "
+                   "LayerDrop are NOT -- the training kernels run eval-mode arithmetic for those ops unless "
+                   "model.encoder_dropout is set (INTEGRATION.md 2c)")
+        warnings.warn(msg, RuntimeWarning, stacklevel=3)
         _WARNED_DROPOUT = True
     P = model._packed()
     bf = model.precision == "bf16"
@@ -191,6 +271,10 @@ def forward_train(model, audio: torch.Tensor, one_hot: torch.Tensor, tmpl: torch
     T = N * fps // 16000
     dev = audio.device
     tp: Dict = {"B": B, "N": N, "T": T, "audio": audio, "one_hot": one_hot}
+    drop = _dropout_plan(model, dev)
+    tp["drop"] = drop
+    ph = drop["hidden"] if drop else 0.0
+    pa = drop["activation"] if drop else 0.0
 
     stats = ops.audio_stats(audio)
     gn = ae.feature_extractor.conv_layers[0].layer_norm
@@ -219,6 +303,8 @@ def forward_train(model, audio: torch.Tensor, one_hot: torch.Tensor, tmpl: torch
     M = B * T
     h0 = torch.empty((M, 768), dtype=dt, device=dev)
     ops.gemm(xi.view(M, 512), P["proj_w"], h0, bias=fp.projection.bias.detach(), backend=be)
+    if drop and drop["feat_proj"] > 0:
+        ops.dropout_apply(h0, drop["feat_proj"], L.DROP_FEAT_PROJ, drop["so"], out=h0)
     if spec_augment_active(model):
         # SpecAugment (ref:src/model/wav2vec.py:149-162): the mask is drawn on the host with the reference's numpy
         # sequence (spec_augment.py), applied and back-propagated by the a2f_spec_mask_* kernels
@@ -230,22 +316,33 @@ def forward_train(model, audio: torch.Tensor, one_hot: torch.Tensor, tmpl: torch
     pre = ops.act_fwd(pc, GELU, resid=h0)
     h = torch.empty((M, 768), dtype=dt, device=dev)
     ops.layernorm(pre, ae.encoder.layer_norm.weight.detach(), ae.encoder.layer_norm.bias.detach(), h)
+    if ph > 0:
+        ops.dropout_apply(h, ph, L.DROP_ENC_IN, drop["so"], out=h)
     tp.update(xi=xi, h0=h0, pc=pc, pre=pre)
     layers = []
-    fuse_ln = bf and getattr(model, "fuse_layernorm", True)
-    for blk, W in zip(ae.encoder.layers, P["layers"]):
+    # the dropout sites of a layer run unfused: GEMM + a2f_dropout_apply (+ the separate LayerNorm)
+    fuse_ln = bf and getattr(model, "fuse_layernorm", True) and ph == 0
+    for li, (blk, W) in enumerate(zip(ae.encoder.layers, P["layers"])):
+        if drop and li in drop["skip"]:
+            layers.append(None)                   # LayerDrop: the layer is the identity and launches nothing
+            continue
         s = {"h_in": h}
         qkv = torch.empty((M, 2304), dtype=dt, device=dev)
         ops.gemm(h, W["qkv_w"], qkv, bias=W["qkv_b"], backend=be)
         att = torch.empty((M, 768), dtype=dt, device=dev)
         lse = torch.empty((B, 12, T), dtype=torch.float32, device=dev)
         att32 = torch.empty((M, 768), dtype=torch.float32, device=dev) if bf else None
-        ops.mha_lse(qkv, att, lse, B, T, out_f32=att32)
+        adrop = (drop["attention"], 8 * li + L.DROP_ATTN_PROB, drop["so"]) if drop and drop["attention"] > 0 else None
+        ops.mha_lse(qkv, att, lse, B, T, out_f32=att32, dropout=adrop)
         pre1 = torch.empty((M, 768), dtype=dt, device=dev)
         h1 = torch.empty((M, 768), dtype=dt, device=dev)
         if fuse_ln:      # LayerNorm in the GEMM epilogue; the pre-LN sum is written once (bf16) for the backward
             ops.gemm_ln(att, W["o_w"], blk.attention.out_proj.bias.detach(), h, blk.layer_norm.weight.detach(),
                         blk.layer_norm.bias.detach(), h1, pre_out=pre1)
+        elif ph > 0:
+            ops.gemm(att, W["o_w"], pre1, bias=blk.attention.out_proj.bias.detach(), backend=be)
+            ops.dropout_apply(pre1, ph, 8 * li + L.DROP_ATTN_OUT, drop["so"], resid=h, out=pre1)
+            ops.layernorm(pre1, blk.layer_norm.weight.detach(), blk.layer_norm.bias.detach(), h1)
         else:
             ops.gemm(att, W["o_w"], pre1, bias=blk.attention.out_proj.bias.detach(), resid=h, backend=be)
             ops.layernorm(pre1, blk.layer_norm.weight.detach(), blk.layer_norm.bias.detach(), h1)
@@ -256,11 +353,17 @@ def forward_train(model, audio: torch.Tensor, one_hot: torch.Tensor, tmpl: torch
         else:
             ops.gemm(h1, W["f1_w"], fpre, bias=blk.feed_forward.intermediate_dense.bias.detach(), backend=be)
             f = ops.act_fwd(fpre, GELU)
+        if pa > 0:
+            ops.dropout_apply(f, pa, 8 * li + L.DROP_FFN_ACT, drop["so"], out=f)
         pre2 = torch.empty((M, 768), dtype=dt, device=dev)
         h = torch.empty((M, 768), dtype=dt, device=dev)
         if fuse_ln:
             ops.gemm_ln(f, W["f2_w"], blk.feed_forward.output_dense.bias.detach(), h1, blk.final_layer_norm.weight.detach(),
                         blk.final_layer_norm.bias.detach(), h, pre_out=pre2)
+        elif ph > 0:
+            ops.gemm(f, W["f2_w"], pre2, bias=blk.feed_forward.output_dense.bias.detach(), backend=be)
+            ops.dropout_apply(pre2, ph, 8 * li + L.DROP_FFN_OUT, drop["so"], resid=h1, out=pre2)
+            ops.layernorm(pre2, blk.final_layer_norm.weight.detach(), blk.final_layer_norm.bias.detach(), h)
         else:
             ops.gemm(f, W["f2_w"], pre2, bias=blk.feed_forward.output_dense.bias.detach(), resid=h1, backend=be)
             ops.layernorm(pre2, blk.final_layer_norm.weight.detach(), blk.final_layer_norm.bias.detach(), h)
@@ -376,24 +479,52 @@ def backward(model, tp: Dict, dout: Optional[torch.Tensor], on_ready=None, dYb: 
         on_ready(0)
 
     # ---- encoder layers ----
+    # dropout (tp["drop"]): the same a2f_dropout_apply with the forward's (seed, offset) snapshot masks a gradient; the
+    # residual branch of a site keeps the unmasked gradient, its Linear (weight, bias, data gradient) gets the masked one
+    drop = tp.get("drop")
+    ph = drop["hidden"] if drop else 0.0
+    pa = drop["activation"] if drop else 0.0
     stage = 0
-    for blk, W, s in zip(reversed(list(ae.encoder.layers)), reversed(PB["layers"]), reversed(tp["layers"])):
+    n_layers = len(tp["layers"])
+    for i, (blk, W, s) in enumerate(zip(reversed(list(ae.encoder.layers)), reversed(PB["layers"]), reversed(tp["layers"]))):
+        li = n_layers - 1 - i
+        stage += 1
+        if s is None:                             # skipped by LayerDrop: no launch, no gradient
+            if on_ready is not None:
+                on_ready(stage)
+            continue
         a, ff = blk.attention, blk.feed_forward
         dpre2 = ops.layernorm_bwd(dh, s["pre2"], blk.final_layer_norm.weight.detach(), _grad(blk.final_layer_norm.weight),
-                                  _grad(blk.final_layer_norm.bias), _grad(ff.output_dense.bias))
-        ops.gemm_wgrad(dpre2, s["f"], _grad(ff.output_dense.weight), backend=be)
+                                  _grad(blk.final_layer_norm.bias), None if ph > 0 else _grad(ff.output_dense.bias))
+        g2 = dpre2
+        if ph > 0:
+            g2 = ops.dropout_apply(dpre2, ph, 8 * li + L.DROP_FFN_OUT, drop["so"])
+            ops.colsum(g2, _grad(ff.output_dense.bias))
+        ops.gemm_wgrad(g2, s["f"], _grad(ff.output_dense.weight), backend=be)
         dfpre = torch.empty((M, 3072), dtype=dt, device=dev)
-        ops.gemm(dpre2, W["f2_t"], dfpre, act=GELU, resid=s["fpre"], resid_mode=L.RESID_DACT, backend=be)
+        if pa > 0:
+            df = torch.empty((M, 3072), dtype=dt, device=dev)
+            ops.gemm(g2, W["f2_t"], df, backend=be)
+            ops.dropout_apply(df, pa, 8 * li + L.DROP_FFN_ACT, drop["so"], out=df)
+            dfpre = ops.act_bwd(df, s["fpre"], GELU)
+            del df
+        else:
+            ops.gemm(g2, W["f2_t"], dfpre, act=GELU, resid=s["fpre"], resid_mode=L.RESID_DACT, backend=be)
         ops.gemm_wgrad(dfpre, s["h1"], _grad(ff.intermediate_dense.weight), backend=be)
         ops.colsum(dfpre, _grad(ff.intermediate_dense.bias))
         dh1 = torch.empty((M, 768), dtype=dt, device=dev)
         ops.gemm(dfpre, W["f1_t"], dh1, resid=dpre2, backend=be)
         dpre1 = ops.layernorm_bwd(dh1, s["pre1"], blk.layer_norm.weight.detach(), _grad(blk.layer_norm.weight),
-                                  _grad(blk.layer_norm.bias), _grad(a.out_proj.bias))
-        ops.gemm_wgrad(dpre1, s["att"], _grad(a.out_proj.weight), backend=be)
+                                  _grad(blk.layer_norm.bias), None if ph > 0 else _grad(a.out_proj.bias))
+        g1 = dpre1
+        if ph > 0:
+            g1 = ops.dropout_apply(dpre1, ph, 8 * li + L.DROP_ATTN_OUT, drop["so"])
+            ops.colsum(g1, _grad(a.out_proj.bias))
+        ops.gemm_wgrad(g1, s["att"], _grad(a.out_proj.weight), backend=be)
         datt = torch.empty((M, 768), dtype=dt, device=dev)
-        ops.gemm(dpre1, W["o_t"], datt, backend=be)
-        dqkv = ops.mha_bwd(s["qkv"], s["att"], datt, s["lse"], B, T, out_f32=s["att32"])
+        ops.gemm(g1, W["o_t"], datt, backend=be)
+        adrop = (drop["attention"], 8 * li + L.DROP_ATTN_PROB, drop["so"]) if drop and drop["attention"] > 0 else None
+        dqkv = ops.mha_bwd(s["qkv"], s["att"], datt, s["lse"], B, T, out_f32=s["att32"], dropout=adrop)
         gw = [_grad(lin.weight) for lin in (a.q_proj, a.k_proj, a.v_proj)]
         gb = [_grad(lin.bias) for lin in (a.q_proj, a.k_proj, a.v_proj)]
         if _adjacent(gw):
@@ -408,11 +539,12 @@ def backward(model, tp: Dict, dout: Optional[torch.Tensor], on_ready=None, dYb: 
             ops.colsum3(dqkv, gb)
         dh = torch.empty((M, 768), dtype=dt, device=dev)
         ops.gemm(dqkv, W["qkv_t"], dh, resid=dpre1, backend=be)
-        stage += 1
         if on_ready is not None:
             on_ready(stage)
 
     # ---- encoder.layer_norm, positional conv, feature projection ----
+    if ph > 0:
+        ops.dropout_apply(dh, ph, L.DROP_ENC_IN, drop["so"], out=dh)
     dpre = ops.layernorm_bwd(dh, tp["pre"], ae.encoder.layer_norm.weight.detach(), _grad(ae.encoder.layer_norm.weight),
                              _grad(ae.encoder.layer_norm.bias))
     pcv = ae.encoder.pos_conv_embed.conv
@@ -425,6 +557,8 @@ def backward(model, tp: Dict, dout: Optional[torch.Tensor], on_ready=None, dYb: 
     dh0 = ops.posconv_dgrad(dpc, PB["pos_bwd"], dpre, B, T, be)
     if tp.get("spec_mask") is not None:
         ops.spec_mask_bwd(dh0, tp["spec_mask"], _grad(ae.masked_spec_embed))
+    if drop and drop["feat_proj"] > 0:
+        ops.dropout_apply(dh0, drop["feat_proj"], L.DROP_FEAT_PROJ, drop["so"], out=dh0)
     fp = ae.feature_projection
     ops.gemm_wgrad(dh0, tp["xi"].view(M, 512), _grad(fp.projection.weight), backend=be)
     ops.colsum(dh0, _grad(fp.projection.bias))

@@ -268,6 +268,17 @@ int a2f_mha_bwd(const void* qkv, const void* out, const void* dout, const float*
 int a2f_mha_bwd_train(const void* qkv, const void* out, const float* out_f32, const void* dout, const float* lse,
                       void* dqkv, int dtype, int B, int T, int H, int D, float scale, void* workspace,
                       size_t workspace_bytes, void* stream);
+/* training with attention dropout (site 8 * layer + A2F_DROP_ATTN_PROB, see "Encoder dropout" below): out = (P o Z/(1-p)) V,
+ * lse stays that of the undropped softmax; Z over the logical tensor [B, H, T, Tp], Tp = ceil(T/8)*8 (padding the key
+ * axis keeps an 8-key group inside one query row).  The backward regenerates Z in registers (dV = (P o Z/(1-p))^T dO,
+ * dP = (dO V^T) o Z/(1-p), dS = P o (dP - delta), delta = rowsum(dO o O) of the dropped O).  A NULL dropout pointer,
+ * p == 0 or a NULL seed_offset_dev is the call without the suffix. */
+struct a2f_dropout_args;
+int a2f_mha_fwd_train_dropout(const void* qkv, void* out, float* lse, float* out_f32, int dtype, int B, int T, int H, int D,
+                              float scale, const struct a2f_dropout_args* dropout, void* stream);
+int a2f_mha_bwd_train_dropout(const void* qkv, const void* out, const float* out_f32, const void* dout, const float* lse,
+                              void* dqkv, int dtype, int B, int T, int H, int D, float scale,
+                              const struct a2f_dropout_args* dropout, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * FaceFormer autoregressive decoder (ref:src/model/faceformer.py:154-185; torch nn.TransformerDecoderLayer
@@ -556,6 +567,42 @@ int a2f_colsum3(const void* x, int dtype, long long ld, long long rows, int seg_
 int a2f_spec_mask_fwd(void* h, int dtype, const unsigned char* mask, const float* embed, long long rows, int cols,
                       void* stream);
 int a2f_spec_mask_bwd(void* dh, int dtype, const unsigned char* mask, float* dembed, long long rows, int cols,
+                      void* stream);
+/* Encoder dropout (training forward of the wav2vec2 encoder; HF modeling_wav2vec2.py train-mode dropout).
+ *
+ * RNG contract -- a keep mask depends only on (seed, offset, site, element index), never on the kernel, tile,
+ * precision or launch that applies it, so a reference implementation can regenerate it exactly:
+ *   generator  Philox4x32-10 (Random123 constants); key = the 64-bit seed (low word first);
+ *              counter = (g lo, g hi, site, offset), where g is a 64-bit group index
+ *   values     one call yields eight 16-bit values: half-word i (i = 0..7) is word i/2 of the output, low half first
+ *   element e  of a site uses call g = e / 8 and half-word e % 8; it is KEPT iff that value >= round(p * 65536) and
+ *              then scaled by 1 / (1 - p) (fp32); dropped elements become 0
+ *   e          the row-major linear index in the site's logical tensor: [B*T, 768] for the hidden sites, [B*T, 3072]
+ *              for the FFN activation, [B, 12, T, Tp] with Tp = ceil(T/8)*8 for the attention probabilities
+ *   site       8 * layer + kind for the per-layer sites (kind: A2F_DROP_ATTN_PROB, A2F_DROP_ATTN_OUT, A2F_DROP_FFN_ACT,
+ *              A2F_DROP_FFN_OUT); A2F_DROP_FEAT_PROJ and A2F_DROP_ENC_IN for the two sites in front of the layers
+ *   seed/offset read from DEVICE memory: seed_offset_dev points at two 64-bit integers {seed, offset}; the low 32 bits
+ *              of offset are used.  A training forward snapshots them for its backward and then advances the offset,
+ *              so a replayed CUDA graph draws fresh masks each step.
+ * A NULL args pointer, a NULL seed_offset_dev or p == 0 means "no dropout". */
+typedef struct a2f_dropout_args {
+    float p;                      /* drop probability in [0, 1) */
+    unsigned site;                /* see the site numbering above */
+    const void* seed_offset_dev;  /* {unsigned long long seed, unsigned long long offset} in device memory, or NULL */
+} a2f_dropout_args;
+
+#define A2F_DROP_ATTN_PROB 0   /* logical tensor [B, H, T, Tp], a2f_mha_fwd_train_dropout / a2f_mha_bwd_train_dropout */
+#define A2F_DROP_ATTN_OUT 1
+#define A2F_DROP_FFN_ACT 2
+#define A2F_DROP_FFN_OUT 3
+#define A2F_DROP_FEAT_PROJ 96
+#define A2F_DROP_ENC_IN 97
+
+/* the keep mask of one site over the first n elements of its logical tensor: mask[e] = 1 (kept) or 0 (dropped) */
+int a2f_dropout_mask(const a2f_dropout_args* args, long long n, unsigned char* mask, void* stream);
+/* y[e] = drop(x[e]) (+ resid[e] when resid is not NULL) over n elements (n % 8 == 0, 16-byte aligned, x / resid / y of
+ * one dtype, A2F_F32 or A2F_BF16; y may alias x or resid).  The backward of a site is the same call on the gradient. */
+int a2f_dropout_apply(const void* x, const void* resid, void* y, int dtype, long long n, const a2f_dropout_args* args,
                       void* stream);
 /* LayerNorm backward over the last dim (C = 512 or 768): x is the saved LayerNorm INPUT.  dgamma / dbeta accumulate;
  * dbias (optional) accumulates the column sums of dx = the bias gradient of the Linear that produced x. */
