@@ -1,12 +1,14 @@
-"""Training step of the two convolutional models on the sm_100a kernels: forward that keeps a tape + explicit backward
-(ref: torch.autograd over ref:src/model/voca.py:38-49 / ref:src/model/audio2face.py:57-66 inside Lightning's
-training_step, ref:src/model/lightning_model.py:150-161).
+"""Training step of the three convolutional models on the sm_100a kernels: forward that keeps a tape + explicit backward
+(ref: torch.autograd over ref:src/model/voca.py:38-49 / ref:src/model/audio2face.py:57-66 / ref:src/model/song2face.py:63-76
+inside Lightning's training_step, ref:src/model/lightning_model.py:150-161).
 
-Audio2Mesh runs its BatchNorms in TRAIN mode here (batch statistics, running-stat update, num_batches_tracked += 1),
-exactly what `model.train()` means in the reference; VOCA has no stochastic or batch-dependent op.  Both models are
-small (1.7 / 131 MFLOP per window), so the whole training path uses the true-fp32 SIMT GEMMs: forward convolutions as
-implicit GEMMs over zero-left-padded channels-last activations, data gradients as gather-segment GEMMs (no col2im),
-weight gradients as transposed-operand GEMMs accumulated straight into `.grad`.
+Audio2Mesh and Song2Face run their BatchNorms in TRAIN mode here (batch statistics, running-stat update,
+num_batches_tracked += 1), exactly what `model.train()` means in the reference; VOCA has no stochastic or batch-dependent
+op, and Song2Face's single-layer LSTMs have no dropout.  The whole training path uses the true-fp32 SIMT GEMMs whatever
+the module's precision: VOCA / Audio2Mesh forward convolutions as implicit GEMMs over zero-left-padded channels-last
+activations with data gradients as gather-segment GEMMs; Song2Face's convolutions as explicit im2col + GEMM with the
+data gradient through the im2col adjoint (a2f_col2im1d); its LSTMs as the input-projection GEMM + the cluster recurrence,
+backward through a2f_lstm_bptt.  Weight gradients are transposed-operand GEMMs accumulated straight into `.grad`.
 """
 from __future__ import annotations
 
@@ -215,7 +217,14 @@ def a2m_forward_train(m, x, one_hot, tmpl):
     ops.gemm(u.valid(), conv_mat(conv.weight), feat, bias=conv.bias.detach(), act=RELU, backend=S, M=bs, K=1024,
              a_row_stride=5 * 256, rows_per_batch=bs)
     tp["art"].append(dict(x=cur, u=u, mr=mr))
-    # ---- output net ----
+    return output_net_forward(m, feat, one_hot, tmpl, tp), tp
+
+
+def output_net_forward(m, feat: torch.Tensor, one_hot: torch.Tensor, tmpl: torch.Tensor, tp: Dict) -> torch.Tensor:
+    """Output MLP + vertex head shared by Audio2Mesh and Song2Face (ref audio2face.py:49-55,65-66 / song2face.py:74-76):
+    cat((feat, one_hot)) -> Linear -> Linear -> Tanh -> Linear -> Linear + template.  feat [bs, 256]; tapes into `tp`."""
+    bs = feat.shape[0]
+    dev = feat.device
     fc = m.output_net
     w0 = fc[0].weight.detach()
     part = torch.empty((bs, 72), dtype=torch.float32, device=dev)
@@ -229,7 +238,22 @@ def a2m_forward_train(m, x, one_hot, tmpl):
     ops.gemm(f1, fc[3].weight.detach(), z, bias=fc[3].bias.detach(), backend=S, ldc=64)
     out = m._vertex_head(z, fc[4].weight, fc[4].bias, tmpl, 1, 50)
     tp.update(feat=feat, one_hot=one_hot, f0=f0, f1pre=f1pre, f1=f1, zhead=z)
-    return out.view(bs, -1, 3), tp
+    return out.view(bs, -1, 3)
+
+
+def output_net_backward(m, tp: Dict, dout: torch.Tensor) -> torch.Tensor:
+    """Backward of output_net_forward.  feat is the ReLU output of the model's last conv: returns the gradient wrt that
+    conv's pre-activation."""
+    fc = m.output_net
+    bs = dout.shape[0]
+    dout = dout.reshape(bs, -1)
+    dz = _head_bwd(dout, tp["zhead"], fc[4])
+    df1 = linear_bwd(dz, tp["f1"], fc[3].weight, fc[3].bias, True)
+    df1pre = ops.act_bwd(df1, tp["f1pre"], TANH)
+    df0 = linear_bwd(df1pre, tp["f0"], fc[1].weight, fc[1].bias, True)
+    linear_bwd(df0, tp["one_hot"], fc[0].weight, fc[0].bias, False, K=m.n_onehot, w_cols=slice(256, 256 + m.n_onehot))
+    dfeat = linear_bwd(df0, tp["feat"], fc[0].weight, None, True, K=256, w_cols=slice(0, 256))
+    return ops.act_bwd(dfeat, tp["feat"], RELU)
 
 
 def _bn_bwd(bn, dy: Pad, y_relu: Optional[Pad], z: Pad, mr) -> Pad:
@@ -240,18 +264,10 @@ def _bn_bwd(bn, dy: Pad, y_relu: Optional[Pad], z: Pad, mr) -> Pad:
 
 
 def a2m_backward(m, tp: Dict, dout: torch.Tensor) -> None:
-    fc = m.output_net
     bs = dout.shape[0]
     dev = dout.device
     CH = m._CH
-    dout = dout.reshape(bs, -1)
-    dz = _head_bwd(dout, tp["zhead"], fc[4])
-    df1 = linear_bwd(dz, tp["f1"], fc[3].weight, fc[3].bias, True)
-    df1pre = ops.act_bwd(df1, tp["f1pre"], TANH)
-    df0 = linear_bwd(df1pre, tp["f0"], fc[1].weight, fc[1].bias, True)
-    linear_bwd(df0, tp["one_hot"], fc[0].weight, fc[0].bias, False, K=m.n_onehot, w_cols=slice(256, 256 + m.n_onehot))
-    dfeat = linear_bwd(df0, tp["feat"], fc[0].weight, None, True, K=256, w_cols=slice(0, 256))
-    dfeat = ops.act_bwd(dfeat, tp["feat"], RELU)
+    dfeat = output_net_backward(m, tp, dout)
     # ---- articulation layer 5: BN -> conv(4x1, s4) -> ReLU ----
     a = tp["art"][4]
     conv, bn = m.articulation_net[13], m.articulation_net[12]
@@ -295,20 +311,164 @@ def a2m_backward(m, tp: Dict, dout: torch.Tensor) -> None:
         dy = conv_k3s2_bwd(a["x"], dzp, m.analysis_net[3 * i], need_dx=i > 0)
 
 
+# ---------------------------------------------------------------------------------------------------------------
+# Song2Face
+# ---------------------------------------------------------------------------------------------------------------
+_S2F_ENC = ((5, 2), (5, 2), (3, 1), (3, 1), (3, 1))         # (taps, pad) of the vocal-encoder convs (stride 2 along W)
+
+
+def _rows(buf: torch.Tensor, C_: int) -> ops.View:
+    """[rows, ld] activation (C_ live columns) as one BatchNorm batch"""
+    buf2 = buf.view(-1, buf.shape[-1])
+    return ops.View(buf2, 0, C_, buf2.shape[0], buf2.stride(0), buf2.numel(), 1)
+
+
+def _conv_fwd(x, outer, ostride, ld, Ci, Li, taps, pad, conv, bn, x_offset=0):
+    """Conv(taps, stride 2, pad) over channels-last x[o*ostride + l*ld + c] as im2col + SIMT GEMM, then BN(train) + ReLU
+    (bn given) or ReLU -> (y [outer*Lo, ldc], tape entry)"""
+    dev = x.device
+    Co = conv.weight.shape[0]
+    K = taps * Ci
+    kpad = (K + 7) // 8 * 8
+    Lo = (Li + 2 * pad - taps) // 2 + 1
+    ldc = (Co + 3) // 4 * 4
+    col = ops.im2col1d(x, outer, ostride, ld, Ci, Li, taps, 2, pad, kpad, False, x_offset=x_offset)
+    wmat = conv_mat(conv.weight)                                   # [Co, tap*Ci + ci]
+    z = torch.empty((outer * Lo, ldc), dtype=torch.float32, device=dev)
+    e = dict(x=x, geom=(outer, ostride, ld, Ci, Li, taps, pad, x_offset), col=col, wmat=wmat, conv=conv, bn=bn, Co=Co, Lo=Lo,
+             ldc=ldc)
+    if bn is None:
+        ops.gemm(col, wmat, z, bias=conv.bias.detach(), act=RELU, backend=S, N=Co, K=K, ldc=ldc)
+        e["y"] = z
+        return z, e
+    ops.gemm(col, wmat, z, bias=conv.bias.detach(), backend=S, N=Co, K=K, ldc=ldc)
+    y = torch.empty_like(z)
+    zv = _rows(z, Co)
+    mr, ss = _bn_fwd(bn, zv)
+    ops.affine_act(zv, zv.like(y), ss, RELU)
+    e.update(z=z, y=y, mr=mr)
+    return y, e
+
+
+def _bn_relu_bwd(e: Dict, dy: torch.Tensor) -> torch.Tensor:
+    """gradient wrt the conv output z of y = ReLU(BN(z)), given dy"""
+    Co, bn = e["Co"], e["bn"]
+    dz = torch.empty_like(e["z"])
+    ops.bn_train_bwd(_rows(dy, Co), _rows(e["y"], Co), _rows(e["z"], Co), e["mr"], bn.weight.detach(), _rows(dz, Co),
+                     _grad(bn.weight), _grad(bn.bias))
+    return dz
+
+
+def _conv_bwd(e: Dict, dz: torch.Tensor, need_dx: bool) -> Optional[torch.Tensor]:
+    """dz: gradient wrt the conv output [outer*Lo, ldc].  Accumulates dW, db; returns dx laid out like the conv input."""
+    outer, ostride, ld, Ci, Li, taps, pad, x_offset = e["geom"]
+    conv, col, Co = e["conv"], e["col"], e["Co"]
+    K = taps * Ci
+    dwp = torch.zeros((Co, K), dtype=torch.float32, device=dz.device)
+    ops.gemm_wgrad(dz, col, dwp, backend=S, N=Co, K=K)
+    ops.add_strided3(dwp, _grad(conv.weight), (Co, taps, Ci), (K, Ci, 1), (Ci * taps, 1, taps))
+    ops.colsum(dz, _grad(conv.bias), cols=Co)
+    if not need_dx:
+        return None
+    wt = ops.transpose_cast(e["wmat"], torch.float32)              # [K, Co]
+    dcol = torch.empty_like(col)
+    ops.gemm(dz, wt, dcol, backend=S, K=Co)
+    return ops.col2im1d(dcol, torch.empty_like(e["x"]), outer, ostride, ld, Ci, Li, taps, 2, pad, x_offset)
+
+
+def lstm_forward_train(lstm: torch.nn.LSTM, x: torch.Tensor):
+    """single-layer batch_first nn.LSTM (hidden 256, zero initial state) on x [B,T,I] -> (h [B,T,256], tape entry)"""
+    B, T, I = x.shape
+    xp = torch.empty((B * T, 1024), dtype=torch.float32, device=x.device)
+    ops.gemm(x.reshape(B * T, I), lstm.weight_ih_l0.detach(), xp, bias=lstm.bias_ih_l0.detach() + lstm.bias_hh_l0.detach(),
+             backend=S)
+    h, gates, cell = ops.lstm_recurrence_train(xp, lstm.weight_hh_l0.detach(), B, T, 256)
+    return h, dict(x=x, h=h, gates=gates, cell=cell)
+
+
+def lstm_backward(lstm: torch.nn.LSTM, e: Dict, dh: torch.Tensor, need_dx: bool = True) -> Optional[torch.Tensor]:
+    """dh [B,T,256] = dL/dh_t from above the layer -> accumulates the four parameter gradients; returns dL/dx [B,T,I]"""
+    x, h = e["x"], e["h"]
+    B, T, I = x.shape
+    H = h.shape[2]
+    da = ops.lstm_bptt(dh.contiguous(), e["gates"], e["cell"], lstm.weight_hh_l0.detach()).view(B * T, 4 * H)
+    if T > 1:                        # dW_hh = sum_{t>=1} da_t^T h_{t-1}: rows t = 1..T-1 of da against rows 0..T-2 of h
+        ops.gemm_wgrad(da, h, _grad(lstm.weight_hh_l0), backend=S, M=B * (T - 1), N=4 * H, K=H, dy_offset=4 * H,
+                       dy_row_stride=4 * H, dy_batch_stride=T * 4 * H, x_row_stride=H, x_batch_stride=T * H, rows_per_batch=T - 1)
+    ops.gemm_wgrad(da, x.reshape(B * T, I), _grad(lstm.weight_ih_l0), backend=S)
+    ops.colsum(da, _grad(lstm.bias_ih_l0))
+    ops.colsum(da, _grad(lstm.bias_hh_l0))
+    if not need_dx:
+        return None
+    wt = ops.transpose_cast(lstm.weight_ih_l0.detach(), torch.float32)            # [I, 4H]
+    dx = torch.empty((B * T, I), dtype=torch.float32, device=x.device)
+    ops.gemm(da, wt, dx, backend=S)
+    return dx.view(B, T, I)
+
+
+def s2f_forward_train(m, x, one_hot, tmpl):
+    bs = x.shape[0]
+    tp: Dict = {"enc": [], "lstm": [], "reg": []}
+    # ---- vocal encoder: conv along W -> BN -> ReLU (ref song2face.py:33-39) ----
+    cur = ops.a2m_assemble(x, one_hot)                              # [B,64,33]; column 0 is an unused zero pad
+    outer, ostride, ld, Ci, Li, xoff = bs * 64, 33, 1, 1, 32, 1
+    for i, (taps, pad) in enumerate(_S2F_ENC):
+        seq = m.vocal_encoder_nn[i]
+        cur, e = _conv_fwd(cur, outer, ostride, ld, Ci, Li, taps, pad, seq[0], seq[1], x_offset=xoff)
+        tp["enc"].append(e)
+        ostride, ld, Ci, Li, xoff = e["Lo"] * e["ldc"], e["ldc"], e["Co"], e["Lo"], 0
+    # ---- two LSTMs over the channel axis: 256 steps of 64 / 256 features (:68-70) ----
+    h = ops.transpose_batched(cur.view(bs, 64, 256))
+    for lstm in (m.vocal_encoder_lstm1, m.vocal_encoder_lstm2):
+        h, e = lstm_forward_train(lstm, h)
+        tp["lstm"].append(e)
+    # ---- bilinear 256 -> 32 resize, regression net conv -> BN -> ReLU, last conv -> ReLU (:54-59, :71-73) ----
+    cur = ops.song2face_resize(h, 32)                               # [B, 32, 256] channels-last
+    outer, ostride, Li = bs, 32 * 256, 32
+    for i in range(4):
+        seq = m.regression_net[i]
+        cur, e = _conv_fwd(cur, outer, ostride, 256, 256, Li, 3, 1 if i < 3 else 0, seq[0], seq[1] if i < 3 else None)
+        tp["reg"].append(e)
+        ostride, Li = e["Lo"] * 256, e["Lo"]
+    return output_net_forward(m, cur, one_hot, tmpl, tp), tp       # cur: [B, 256] (one output row per window)
+
+
+def s2f_backward(m, tp: Dict, dout: torch.Tensor) -> None:
+    bs = dout.shape[0]
+    dz = output_net_backward(m, tp, dout)
+    for i in (3, 2, 1, 0):
+        e = tp["reg"][i]
+        if i < 3:
+            dz = _bn_relu_bwd(e, dy)
+        dy = _conv_bwd(e, dz, need_dx=True)
+    dh = ops.song2face_resize_bwd(dy.view(bs, 32, 256), 256)
+    dh = lstm_backward(m.vocal_encoder_lstm2, tp["lstm"][1], dh)
+    dx = lstm_backward(m.vocal_encoder_lstm1, tp["lstm"][0], dh)   # [B, 256 steps, 64 features]
+    dy = ops.transpose_batched(dx)                                 # [B, 64, 256] = the last vocal-encoder layer's rows
+    for i in (4, 3, 2, 1, 0):
+        e = tp["enc"][i]
+        dz = _bn_relu_bwd(e, dy)
+        dy = _conv_bwd(e, dz, need_dx=i > 0)
+
+
+_TRAIN_FNS = {"voca": (voca_forward_train, voca_backward), "audio2mesh": (a2m_forward_train, a2m_backward),
+              "song2face": (s2f_forward_train, s2f_backward)}
+
+
 class ConvModelTrainFn(torch.autograd.Function):
-    """Glue to torch.autograd for Voca / Audio2Mesh (same scheme as training.FaceformerTrainFn): every parameter is an input
-    of the Function and its gradient an output of backward(), so AccumulateGrad / torch DDP hooks fire per parameter."""
+    """Glue to torch.autograd for Voca / Audio2Mesh / Song2Face (same scheme as training.FaceformerTrainFn): every parameter
+    is an input of the Function and its gradient an output of backward(), so AccumulateGrad / torch DDP hooks fire per
+    parameter."""
 
     @staticmethod
     def forward(ctx, model, kind, x, one_hot, tmpl, *params):
-        fwd = voca_forward_train if kind == "voca" else a2m_forward_train
-        out, tape = fwd(model, x, one_hot, tmpl)
+        out, tape = _TRAIN_FNS[kind][0](model, x, one_hot, tmpl)
         ctx.model, ctx.tape, ctx.kind = model, tape, kind
         return out
 
     @staticmethod
     def backward(ctx, dout):
-        bwd = voca_backward if ctx.kind == "voca" else a2m_backward
+        bwd = _TRAIN_FNS[ctx.kind][1]
         with collect_grads(list(ctx.model.parameters())) as sink:
             bwd(ctx.model, ctx.tape, dout.contiguous().float())
         ctx.tape = None

@@ -230,6 +230,11 @@ _SIGNATURES = {
     "a2f_transpose_batched": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "a2f_lstm_recurrence": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "a2f_song2face_resize": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "a2f_lstm_recurrence_train": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
+    "a2f_lstm_bptt": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
+    "a2f_col2im1d": (c_int, [c_void_p, c_ll, c_ll, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p,
+                             c_void_p]),
+    "a2f_song2face_resize_bwd": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "a2f_adam_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_float, c_float, c_float, c_float, c_float,
                               c_int, c_float, c_void_p]),
     "a2f_adam_step_bf16g": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_float, c_float, c_float, c_float, c_float,

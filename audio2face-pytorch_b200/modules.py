@@ -373,8 +373,10 @@ class Audio2Mesh(_A2FModule):
 
 # ----------------------------------------------------------------------------------------------------------------
 class Song2Face(_A2FModule):
-    """Drop-in for ref:src/model/song2face.py:5-72 (registry entry "song2face", ref:src/model/lightning_model.py:50-58),
-    inference (eval-mode BatchNorm).  Same sub-module names, so the state_dict keys (and their order) are the reference's.
+    """Drop-in for ref:src/model/song2face.py:5-72 (registry entry "song2face", ref:src/model/lightning_model.py:50-58).
+    Same sub-module names, so the state_dict keys (and their order) are the reference's.  eval(): the inference path below
+    (eval-mode BatchNorm).  train(): the training step of conv_training.py (batch-statistics BatchNorm, LSTM
+    backpropagation through time in a2f_lstm_bptt), like Audio2Mesh.
 
     Every convolution is an explicit im2col (csrc/a2m.cu) + a2f_gemm with the folded BatchNorm / bias / ReLU epilogue; the
     two LSTMs run over the CHANNEL axis like the reference (256 steps of 64 / 256 features): input projections of all steps
@@ -452,12 +454,21 @@ class Song2Face(_A2FModule):
 
     def forward(self, x, one_hot, template, **kwargs):
         self._need_cuda(x, one_hot, template)
-        if self.training or (torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())):
-            raise L.A2FError("Song2Face: only the inference path (eval mode, torch.no_grad()) is built on the sm_100a kernels")
         bs = x.size(0)
         x = x.contiguous().float()
         one_hot = one_hot.contiguous().float()
         tmpl = template.reshape(bs, -1).contiguous().float()
+        grad = torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())
+        if self.training:
+            # model.train(): BatchNorm uses batch statistics and updates its running stats; true-fp32 convolutions and LSTMs
+            # whatever the precision, the vertex head follows it as for Audio2Mesh (conv_training.py)
+            from . import conv_training
+            if grad:
+                return conv_training.ConvModelTrainFn.run(self, "song2face", x, one_hot, tmpl)
+            return conv_training.s2f_forward_train(self, x, one_hot, tmpl)[0]
+        if grad:
+            raise L.A2FError("Song2Face: gradients with eval-mode (frozen) BatchNorm are not built; call .train() or "
+                             "run under torch.no_grad()")
         P = self._packed()
         bf = self.precision == "bf16"
         cur = ops.a2m_assemble(x, one_hot)                                   # [B,64,33]; column 0 is an unused zero pad

@@ -447,6 +447,19 @@ def im2col1d(x: torch.Tensor, outer: int, outer_stride: int, ld: int, C_: int, L
     return out
 
 
+def col2im1d(dcol: torch.Tensor, dx: torch.Tensor, outer: int, outer_stride: int, ld: int, C_: int, L_: int, taps: int, stride: int,
+             pad: int, x_offset: int = 0) -> torch.Tensor:
+    """adjoint of im2col1d(split=False): writes every valid element (l < L, c < C) of dx, laid out like im2col1d's x"""
+    _dev(dcol, dx)
+    L_out = (L_ + 2 * pad - taps) // stride + 1
+    if dcol.dim() != 2 or dcol.shape[0] != outer * L_out or dcol.stride(0) != dcol.shape[1] or \
+            dx.numel() < x_offset + (outer - 1) * outer_stride + (L_ - 1) * ld + C_:
+        raise L.A2FError("col2im1d: dcol must be a dense [outer*L_out, kpad] matrix and dx must hold the strided layout")
+    L.check(L.load().a2f_col2im1d(dx.data_ptr() + x_offset * 4, outer, outer_stride, ld, C_, L_, taps, stride, pad, None, None,
+                                  dcol.shape[1], dcol.data_ptr(), _stream()), "a2f_col2im1d")
+    return dx
+
+
 def transpose_batched(x: torch.Tensor) -> torch.Tensor:
     """[B, R, C] fp32 -> [B, C, R]"""
     _dev(x)
@@ -474,6 +487,40 @@ def song2face_resize(h: torch.Tensor, out_h: int) -> torch.Tensor:
     out = torch.empty((B, out_h, T), dtype=torch.float32, device=h.device)
     L.check(L.load().a2f_song2face_resize(h.data_ptr(), B, T, hid, out_h, out.data_ptr(), _stream()), "a2f_song2face_resize")
     return out
+
+
+def song2face_resize_bwd(dout: torch.Tensor, hidden: int) -> torch.Tensor:
+    """adjoint of song2face_resize: dout [B, out_h, T] -> dh [B, T, hidden]"""
+    _dev(dout)
+    B, out_h, T = dout.shape
+    dh = torch.empty((B, T, hidden), dtype=torch.float32, device=dout.device)
+    L.check(L.load().a2f_song2face_resize_bwd(dout.data_ptr(), B, T, hidden, out_h, dh.data_ptr(), _stream()),
+            "a2f_song2face_resize_bwd")
+    return dh
+
+
+def lstm_recurrence_train(xp: torch.Tensor, whh: torch.Tensor, B: int, T: int, hidden: int):
+    """training forward of the recurrence: xp [B,T,4H], whh = W_hh [4H,H] -> (h [B,T,H], gates [B,T,4H], c [B,T,H])"""
+    _dev(xp, whh)
+    h = torch.empty((B, T, hidden), dtype=torch.float32, device=xp.device)
+    gates = torch.empty((B, T, 4 * hidden), dtype=torch.float32, device=xp.device)
+    cell = torch.empty((B, T, hidden), dtype=torch.float32, device=xp.device)
+    L.check(L.load().a2f_lstm_recurrence_train(xp.data_ptr(), whh.data_ptr(), h.data_ptr(), gates.data_ptr(), cell.data_ptr(), B, T,
+                                               hidden, _stream()), "a2f_lstm_recurrence_train")
+    return h, gates, cell
+
+
+def lstm_bptt(dh_out: torch.Tensor, gates: torch.Tensor, cell: torch.Tensor, whh: torch.Tensor) -> torch.Tensor:
+    """dh_out [B,T,H], the saved gates / c, W_hh [4H,H] -> dgates [B,T,4H] (gradient of the pre-activation gates)"""
+    _dev(dh_out, gates, cell, whh)
+    B, T, hidden = cell.shape
+    for t, shape in ((dh_out, (B, T, hidden)), (gates, (B, T, 4 * hidden)), (whh, (4 * hidden, hidden))):
+        if tuple(t.shape) != shape or not t.is_contiguous():
+            raise L.A2FError(f"lstm_bptt: expected a contiguous tensor of shape {shape}, got {tuple(t.shape)}")
+    dgates = torch.empty((B, T, 4 * hidden), dtype=torch.float32, device=cell.device)
+    L.check(L.load().a2f_lstm_bptt(dh_out.data_ptr(), gates.data_ptr(), cell.data_ptr(), whh.data_ptr(), dgates.data_ptr(), B, T,
+                                   hidden, _stream()), "a2f_lstm_bptt")
+    return dgates
 
 
 def a2m_mlp(feat: torch.Tensor, extra: torch.Tensor, fc0, fc1, fc2, ldz: int = 64) -> torch.Tensor:

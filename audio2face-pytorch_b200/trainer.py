@@ -403,7 +403,7 @@ class GraphedTrainStep:
 
 
 class ConvModelTrainer:
-    """Training step of the convolutional models (Voca / Audio2Mesh) with an optional feature extractor in front:
+    """Training step of the convolutional models (Voca / Audio2Mesh / Song2Face) with an optional feature extractor in front:
     the reference's default configuration (ref:config.yaml: modelname audio2mesh, feature_extractor mfcc, batch 128)
     as Lightning runs it (ref:src/model/lightning_model.py:111-117 forward, :145-161 training_step, :209-213 Adam).
 

@@ -443,6 +443,30 @@ int a2f_lstm_recurrence(const float* xp, const float* whh_t, const float* whh_n,
 /* out[b, i, t] = bilinear resize (align_corners = False) of h[b, t, :] from `hidden` to out_h samples: ref song2face.py:65-66
  * F.interpolate(x.unsqueeze(3), size=(32, 1)) written channels-last [B, out_h, T] for the regression convs */
 int a2f_song2face_resize(const float* h, int B, int T, int hidden, int out_h, float* out, void* stream);
+/* ---- Song2Face training step (model.train(); conv_training.py).  All fp32, hidden must be 256, any B >= 1 (8-CTA
+ * clusters of 8 sequences; a partly filled cluster ignores the missing sequences). ----
+ * a2f_lstm_recurrence_train: the recurrence of a2f_lstm_recurrence on the cluster kernel for every B, whh_n = W_hh
+ *   [4*hidden, hidden]; hout [B, T, hidden] as there (bit-identical from B = 4 on, where inference runs the same kernel),
+ *   and per step the post-activation gates [B, T, 4*hidden] (i, f, g, o = sigmoid, sigmoid, tanh, sigmoid) and the cell
+ *   state c_t [B, T, hidden] that a2f_lstm_bptt reads. */
+int a2f_lstm_recurrence_train(const float* xp, const float* whh_n, float* hout, float* gates, float* cell, int B, int T, int hidden,
+                              void* stream);
+/* a2f_lstm_bptt: backpropagation through time of that LSTM.  dh_out [B, T, hidden] = dL/dh_t from above the layer;
+ *   gates / cell as saved by a2f_lstm_recurrence_train; -> dgates [B, T, 4*hidden] = dL/d(pre-activation gates), i.e.
+ *   dL/dxp.  For t = T-1 .. 0 with dh = dh_out_t + W_hh^T da_{t+1}, dc carried from t+1, c_{-1} = 0:
+ *     tc = tanh(c_t); dc += dh o (1 - tc^2); da = (dc g i(1-i), dc c_{t-1} f(1-f), dc i (1-g^2), dh tc o(1-o)); dc <- dc f.
+ *   The weight, bias and input gradients follow from dgates by GEMMs.  Deterministic (no atomics). */
+int a2f_lstm_bptt(const float* dh_out, const float* gates, const float* cell, const float* whh_n, float* dgates, int B, int T,
+                  int hidden, void* stream);
+/* a2f_col2im1d: adjoint of a2f_im2col1d with the same argument list (x becomes the output dx, out the input dcol):
+ *   dx[o*outer_stride + l*ld + c] = sum over (lo, tap) with lo*stride - pad + tap = l of dcol[o*L_out + lo, tap*C + c]
+ *   (times scale[c] when scale != NULL; shift does not enter the adjoint).  Every element l < L, c < C of dx is written
+ *   (gathered, deterministic); columns c >= C of a row are left untouched. */
+int a2f_col2im1d(float* dx, long long outer, long long outer_stride, int ld, int C, int L, int taps, int stride, int pad,
+                 const float* scale, const float* shift, int kpad, const float* dcol, void* stream);
+/* a2f_song2face_resize_bwd: adjoint of a2f_song2face_resize: dout [B, out_h, T] -> dh [B, T, hidden], every column written
+ *   (zeros where no output sample reads a hidden unit); gathered, deterministic. */
+int a2f_song2face_resize_bwd(const float* dout, int B, int T, int hidden, int out_h, float* dh, void* stream);
 /* fused output MLP of Audio2Mesh (ref:src/model/audio2face.py:49-55 minus the vertex head):
  *   z[r, :n2] = W2 tanh(W1 (W0 [feat[r, :k_feat] ; extra[r, :k_extra]] + b0) + b1) + b2,  z[r, n2:ldz] = 0
  * all fp32, row-major weights [n_out, n_in]; every width <= 512. */
