@@ -2,10 +2,12 @@
 (ref: torch.autograd over ref:src/model/voca.py:38-49 / ref:src/model/audio2face.py:57-66 / ref:src/model/song2face.py:63-76
 inside Lightning's training_step, ref:src/model/lightning_model.py:150-161).
 
-Audio2Mesh and Song2Face run their BatchNorms in TRAIN mode here (batch statistics, running-stat update,
-num_batches_tracked += 1), exactly what `model.train()` means in the reference; VOCA has no stochastic or batch-dependent
-op, and Song2Face's single-layer LSTMs have no dropout.  The whole training path uses the true-fp32 SIMT GEMMs whatever
-the module's precision: VOCA / Audio2Mesh forward convolutions as implicit GEMMs over zero-left-padded channels-last
+Audio2Mesh and Song2Face run each BatchNorm by torch's per-layer rule: one in train() uses batch statistics and updates
+its running statistics (num_batches_tracked += 1), exactly what `model.train()` means in the reference; one put in eval()
+inside a train() model ("frozen", the usual fine-tuning recipe) normalises with its running statistics, leaves them
+untouched and passes gradients through that fixed affine map (`_bn_fwd` decides, the tape carries the mode to the
+backward).  VOCA has no stochastic or batch-dependent op, and Song2Face's single-layer LSTMs have no dropout.  The
+whole training path uses the true-fp32 SIMT GEMMs whatever the module's precision: VOCA / Audio2Mesh forward convolutions as implicit GEMMs over zero-left-padded channels-last
 activations with data gradients as gather-segment GEMMs; Song2Face's convolutions as explicit im2col + GEMM with the
 data gradient through the im2col adjoint (a2f_col2im1d); its LSTMs as the input-projection GEMM + the cluster recurrence,
 backward through a2f_lstm_bptt.  Weight gradients are transposed-operand GEMMs accumulated straight into `.grad`.
@@ -162,13 +164,26 @@ def voca_backward(m, tp: Dict, dout: torch.Tensor) -> None:
 # Audio2Mesh
 # ---------------------------------------------------------------------------------------------------------------
 def _bn_fwd(bn: torch.nn.BatchNorm2d, src: ops.View):
-    """train-mode statistics of `src` + running-stat update (momentum None = cumulative average is not used by the
-    reference: nn.BatchNorm2d defaults, momentum 0.1)."""
+    """One BatchNorm of a training forward, by torch's per-layer rule (`bn.training`) -> (tape, scale_shift).
+    train(): statistics of `src` + running-stat update (momentum None = cumulative average is not used by the reference:
+    nn.BatchNorm2d defaults, momentum 0.1).  eval() ("frozen", the fine-tuning recipe): the running statistics, only
+    read.  The tape is (mean_rstd, frozen): the backward follows the mode of the forward, whatever `bn.training` says by
+    then."""
+    if not bn.training:
+        mr, ss = ops.bn_frozen_stats(bn.weight.detach(), bn.bias.detach(), bn.eps, bn.running_mean, bn.running_var)
+        return (mr, True), ss
     mr, ss = ops.bn_train_stats(src, bn.weight.detach(), bn.bias.detach(), bn.eps, bn.momentum, bn.running_mean, bn.running_var)
     bn.num_batches_tracked += 1
     for t in (bn.running_mean, bn.running_var):          # written through raw pointers: invalidate derived-weight caches
         torch.autograd.graph.increment_version(t)
-    return mr, ss
+    return (mr, False), ss
+
+
+def _bn_bwd_into(bn: torch.nn.BatchNorm2d, tape, dy: ops.View, y_relu: Optional[ops.View], z: ops.View, dz: ops.View):
+    """dz = gradient wrt the BatchNorm input, dgamma / dbeta accumulated, in the mode `_bn_fwd` taped"""
+    mr, frozen = tape
+    (ops.bn_frozen_bwd if frozen else ops.bn_train_bwd)(dy, y_relu, z, mr, bn.weight.detach(), dz, _grad(bn.weight),
+                                                        _grad(bn.bias))
 
 
 def a2m_forward_train(m, x, one_hot, tmpl):
@@ -189,34 +204,34 @@ def a2m_forward_train(m, x, one_hot, tmpl):
             ops.gemm(cur.buf, wmat, z.buf, bias=conv.bias.detach(), backend=S, M=bs * 64, K=3 * CH[4], a_row_stride=3 * CH[4],
                      a_batch_stride=64 * 3 * CH[4], rows_per_batch=64, ldc=256, c_batch_stride=65 * 256, c_offset=256)
             y = z.zeros_like()
-        mr, ss = _bn_fwd(bn, z.view())
+        bt, ss = _bn_fwd(bn, z.view())
         ops.affine_act(z.view(), y.view(), ss, RELU)
-        tp["ana"].append(dict(x=cur, z=z, y=y, mr=mr))
+        tp["ana"].append(dict(x=cur, z=z, y=y, bt=bt))
         cur = y
     # ---- articulation net: conv along H ----
     for ci, bi in ((0, 1), (3, 4), (6, 7)):                        # conv -> BN -> ReLU (ref audio2face.py:31-40)
         conv, bn = m.articulation_net[ci], m.articulation_net[bi]
         z = conv_k3s2_fwd(cur, conv_mat(conv.weight), conv.bias.detach(), NONE)
         y = z.zeros_like()
-        mr, ss = _bn_fwd(bn, z.view())
+        bt, ss = _bn_fwd(bn, z.view())
         ops.affine_act(z.view(), y.view(), ss, RELU)
-        tp["art"].append(dict(x=cur, z=z, y=y, mr=mr))
+        tp["art"].append(dict(x=cur, z=z, y=y, bt=bt))
         cur = y
     bn, conv = m.articulation_net[9], m.articulation_net[10]       # BN -> conv -> ReLU (ref audio2face.py:41-43)
-    mr, ss = _bn_fwd(bn, cur.view())
+    bt, ss = _bn_fwd(bn, cur.view())
     u = cur.zeros_like()
     ops.affine_act(cur.view(), u.view(), ss, NONE)
     y = conv_k3s2_fwd(u, conv_mat(conv.weight), conv.bias.detach(), RELU)
-    tp["art"].append(dict(x=cur, u=u, y=y, mr=mr))
+    tp["art"].append(dict(x=cur, u=u, y=y, bt=bt))
     cur = y                                                        # [bs, 4(+1), 256]
     bn, conv = m.articulation_net[12], m.articulation_net[13]      # BN -> conv(4x1, stride 4) -> ReLU (:44-46)
-    mr, ss = _bn_fwd(bn, cur.view())
+    bt, ss = _bn_fwd(bn, cur.view())
     u = cur.zeros_like()
     ops.affine_act(cur.view(), u.view(), ss, NONE)
     feat = torch.empty((bs, 256), dtype=torch.float32, device=dev)
     ops.gemm(u.valid(), conv_mat(conv.weight), feat, bias=conv.bias.detach(), act=RELU, backend=S, M=bs, K=1024,
              a_row_stride=5 * 256, rows_per_batch=bs)
-    tp["art"].append(dict(x=cur, u=u, mr=mr))
+    tp["art"].append(dict(x=cur, u=u, bt=bt))
     return output_net_forward(m, feat, one_hot, tmpl, tp), tp
 
 
@@ -256,10 +271,9 @@ def output_net_backward(m, tp: Dict, dout: torch.Tensor) -> torch.Tensor:
     return ops.act_bwd(dfeat, tp["feat"], RELU)
 
 
-def _bn_bwd(bn, dy: Pad, y_relu: Optional[Pad], z: Pad, mr) -> Pad:
+def _bn_bwd(bn, dy: Pad, y_relu: Optional[Pad], z: Pad, bt) -> Pad:
     dz = z.zeros_like()
-    ops.bn_train_bwd(dy.view(), y_relu.view() if y_relu is not None else None, z.view(), mr, bn.weight.detach(), dz.view(),
-                     _grad(bn.weight), _grad(bn.bias))
+    _bn_bwd_into(bn, bt, dy.view(), y_relu.view() if y_relu is not None else None, z.view(), dz.view())
     return dz
 
 
@@ -278,22 +292,22 @@ def a2m_backward(m, tp: Dict, dout: torch.Tensor) -> None:
     du = a["u"].zeros_like()
     wt = ops.transpose_cast(conv_mat(conv.weight), torch.float32)                      # [1024, 256]
     ops.gemm(dfeat, wt, du.buf, backend=S, ldc=5 * 256, c_offset=256)
-    dy = _bn_bwd(bn, du, None, a["x"], a["mr"])
+    dy = _bn_bwd(bn, du, None, a["x"], a["bt"])
     # ---- articulation layer 4: BN -> conv -> ReLU ----
     a = tp["art"][3]
     conv, bn = m.articulation_net[10], m.articulation_net[9]
     dzp = Pad(dy.nb, dy.L, dy.C, dev, buf=ops.act_bwd(dy.buf, a["y"].buf, RELU))
     du = conv_k3s2_bwd(a["u"], dzp, conv, True)
-    dy = _bn_bwd(bn, du, None, a["x"], a["mr"])
+    dy = _bn_bwd(bn, du, None, a["x"], a["bt"])
     # ---- articulation layers 3..1: conv -> BN -> ReLU ----
     for j, (ci, bi) in zip((2, 1, 0), ((6, 7), (3, 4), (0, 1))):
         a = tp["art"][j]
-        dzp = _bn_bwd(m.articulation_net[bi], dy, a["y"], a["z"], a["mr"])
+        dzp = _bn_bwd(m.articulation_net[bi], dy, a["y"], a["z"], a["bt"])
         dy = conv_k3s2_bwd(a["x"], dzp, m.articulation_net[ci], True)
     # ---- analysis layer 5 (W 2 -> 1): a Linear 3*243 -> 256 per (b, h) ----
     a = tp["ana"][4]
     conv, bn = m.analysis_net[12], m.analysis_net[13]
-    dzp = _bn_bwd(bn, dy, a["y"], a["z"], a["mr"])
+    dzp = _bn_bwd(bn, dy, a["y"], a["z"], a["bt"])
     ops.colsum(dzp.buf.view(-1, 256), _grad(conv.bias))
     Ci = CH[4]
     dwp = torch.zeros((256, 3 * Ci), dtype=torch.float32, device=dev)
@@ -307,7 +321,7 @@ def a2m_backward(m, tp: Dict, dout: torch.Tensor) -> None:
     # ---- analysis layers 4..1 ----
     for i in (3, 2, 1, 0):
         a = tp["ana"][i]
-        dzp = _bn_bwd(m.analysis_net[3 * i + 1], dy, a["y"], a["z"], a["mr"])
+        dzp = _bn_bwd(m.analysis_net[3 * i + 1], dy, a["y"], a["z"], a["bt"])
         dy = conv_k3s2_bwd(a["x"], dzp, m.analysis_net[3 * i], need_dx=i > 0)
 
 
@@ -324,7 +338,7 @@ def _rows(buf: torch.Tensor, C_: int) -> ops.View:
 
 
 def _conv_fwd(x, outer, ostride, ld, Ci, Li, taps, pad, conv, bn, x_offset=0):
-    """Conv(taps, stride 2, pad) over channels-last x[o*ostride + l*ld + c] as im2col + SIMT GEMM, then BN(train) + ReLU
+    """Conv(taps, stride 2, pad) over channels-last x[o*ostride + l*ld + c] as im2col + SIMT GEMM, then BN + ReLU
     (bn given) or ReLU -> (y [outer*Lo, ldc], tape entry)"""
     dev = x.device
     Co = conv.weight.shape[0]
@@ -344,9 +358,9 @@ def _conv_fwd(x, outer, ostride, ld, Ci, Li, taps, pad, conv, bn, x_offset=0):
     ops.gemm(col, wmat, z, bias=conv.bias.detach(), backend=S, N=Co, K=K, ldc=ldc)
     y = torch.empty_like(z)
     zv = _rows(z, Co)
-    mr, ss = _bn_fwd(bn, zv)
+    bt, ss = _bn_fwd(bn, zv)
     ops.affine_act(zv, zv.like(y), ss, RELU)
-    e.update(z=z, y=y, mr=mr)
+    e.update(z=z, y=y, bt=bt)
     return y, e
 
 
@@ -354,8 +368,7 @@ def _bn_relu_bwd(e: Dict, dy: torch.Tensor) -> torch.Tensor:
     """gradient wrt the conv output z of y = ReLU(BN(z)), given dy"""
     Co, bn = e["Co"], e["bn"]
     dz = torch.empty_like(e["z"])
-    ops.bn_train_bwd(_rows(dy, Co), _rows(e["y"], Co), _rows(e["z"], Co), e["mr"], bn.weight.detach(), _rows(dz, Co),
-                     _grad(bn.weight), _grad(bn.bias))
+    _bn_bwd_into(bn, e["bt"], _rows(dy, Co), _rows(e["y"], Co), _rows(e["z"], Co), _rows(dz, Co))
     return dz
 
 

@@ -66,22 +66,30 @@ __global__ void __launch_bounds__(256) bn_moments_kernel(const float* __restrict
 
 // mean / rstd, the fused scale / shift of y = gamma*(x-mean)*rstd + beta, and the running-stat update
 // (torch BatchNorm2d train mode: biased variance normalises, unbiased variance feeds running_var, momentum 0.1)
+// FROZEN (eval-mode BatchNorm): mean / var are the running statistics, which are only read; `sums` is unused
+template <bool FROZEN>
 __global__ void bn_finalize_kernel(const double* __restrict__ sums, int C, double n, const float* __restrict__ gamma,
                                    const float* __restrict__ beta, float eps, float momentum, float* __restrict__ running_mean,
                                    float* __restrict__ running_var, float* __restrict__ mean_rstd,
                                    float* __restrict__ scale_shift) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= C) return;
-    const double mean = sums[c] / n;
-    double var = sums[C + c] / n - mean * mean;
-    if (var < 0.0) var = 0.0;
+    double mean, var;
+    if (FROZEN) {
+        mean = running_mean[c];
+        var = running_var[c];
+    } else {
+        mean = sums[c] / n;
+        var = sums[C + c] / n - mean * mean;
+        if (var < 0.0) var = 0.0;
+    }
     const double rstd = 1.0 / sqrt(var + (double)eps);
     mean_rstd[c] = (float)mean;
     mean_rstd[C + c] = (float)rstd;
     const float sc = (float)((double)gamma[c] * rstd);
     scale_shift[c] = sc;
     scale_shift[C + c] = (float)((double)beta[c] - mean * (double)gamma[c] * rstd);
-    if (running_mean != nullptr) {
+    if (!FROZEN && running_mean != nullptr) {
         running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)mean;
         const double unbiased = n > 1.0 ? var * n / (n - 1.0) : var;
         running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unbiased;
@@ -143,6 +151,8 @@ __global__ void __launch_bounds__(256) bn_bwd_reduce_kernel(const float* __restr
 }
 
 // dz = gamma*rstd * (dy_eff - mean(dy_eff) - xhat * mean(dy_eff * xhat));  dgamma += sum dy_eff*xhat, dbeta += sum dy_eff
+// FROZEN (eval-mode BatchNorm, mean / rstd from the running statistics, so constants): dz = gamma*rstd * dy_eff
+template <bool FROZEN>
 __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(const float* __restrict__ dy, const float* __restrict__ y,
                                                            const float* __restrict__ z, const float* __restrict__ mean_rstd,
                                                            const float* __restrict__ gamma, const double* __restrict__ sums,
@@ -164,9 +174,13 @@ __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(const float* __restri
         float g = dy[off];
         if (y != nullptr && !(y[off] > 0.f)) g = 0.f;
         const float rstd = mean_rstd[C + c];
-        const float xh = (z[off] - mean_rstd[c]) * rstd;
-        const float m1 = (float)(sums[c] / n), m2 = (float)(sums[C + c] / n);
-        dz[off] = gamma[c] * rstd * (g - m1 - xh * m2);
+        if (FROZEN) {
+            dz[off] = gamma[c] * rstd * g;
+        } else {
+            const float xh = (z[off] - mean_rstd[c]) * rstd;
+            const float m1 = (float)(sums[c] / n), m2 = (float)(sums[C + c] / n);
+            dz[off] = gamma[c] * rstd * (g - m1 - xh * m2);
+        }
     }
 }
 
@@ -174,6 +188,29 @@ static int ew_blocks(long long n) {
     long long b = (n + 255) / 256;
     const long long cap = 8LL * sm_count();
     return (int)(b > cap ? cap : (b < 1 ? 1 : b));
+}
+
+// a2f_bn_train_bwd / a2f_bn_frozen_bwd after argument checks: the same two launches (reduce, apply), differing only in
+// the apply instantiation
+template <bool FROZEN>
+static int bn_bwd_launch(const float* dy, const float* y_relu, const float* z, const float* mean_rstd, const float* gamma,
+                         int C, long long rows_per_batch, long long ld, long long batch_stride, long long batches,
+                         float* dz, float* dgamma, float* dbeta, void* workspace, void* stream) {
+    cudaStream_t s = as_stream(stream);
+    double* sums = static_cast<double*>(workspace);
+    A2F_CHECK_CUDA(cudaMemsetAsync(sums, 0, (size_t)2 * C * sizeof(double), s));
+    const long long rows = batches * rows_per_batch;
+    long long gy = (rows + 63) / 64;
+    if (gy > 256) gy = 256;
+    bn_bwd_reduce_kernel<<<dim3((C + 31) / 32, (unsigned)gy), 256, 0, s>>>(dy, y_relu, z, mean_rstd, C, rows_per_batch, ld,
+                                                                            batch_stride, batches, sums);
+    A2F_CHECK_LAUNCH("bn_bwd_reduce_kernel");
+    bn_bwd_apply_kernel<FROZEN><<<ew_blocks(rows * C), 256, 0, s>>>(dy, y_relu, z, mean_rstd, gamma, sums, (double)rows, C,
+                                                                     rows_per_batch, ld, batch_stride, batches, dz, dgamma,
+                                                                     dbeta);
+    A2F_CHECK_LAUNCH("bn_bwd_apply_kernel");
+    count_launch(2);
+    return A2F_OK;
 }
 
 }  // namespace a2f
@@ -211,10 +248,24 @@ int a2f_bn_train_stats(const float* x, int C, long long rows_per_batch, long lon
     if (gy > 256) gy = 256;
     bn_moments_kernel<<<dim3((C + 31) / 32, (unsigned)gy), 256, 0, s>>>(x, C, rows_per_batch, ld, batch_stride, batches, sums);
     A2F_CHECK_LAUNCH("bn_moments_kernel");
-    bn_finalize_kernel<<<(C + 127) / 128, 128, 0, s>>>(sums, C, (double)rows, gamma, beta, eps, momentum, running_mean,
-                                                        running_var, mean_rstd, scale_shift);
+    bn_finalize_kernel<false><<<(C + 127) / 128, 128, 0, s>>>(sums, C, (double)rows, gamma, beta, eps, momentum,
+                                                               running_mean, running_var, mean_rstd, scale_shift);
     A2F_CHECK_LAUNCH("bn_finalize_kernel");
     count_launch(2);
+    return A2F_OK;
+}
+
+int a2f_bn_frozen_stats(const float* gamma, const float* beta, float eps, const float* running_mean,
+                        const float* running_var, int C, float* mean_rstd, float* scale_shift, void* stream) {
+    int rc = require_sm100();
+    if (rc != A2F_OK) return rc;
+    A2F_REQUIRE(gamma && beta && running_mean && running_var && mean_rstd && scale_shift && C > 0,
+                "a2f_bn_frozen_stats: bad arguments");
+    bn_finalize_kernel<true><<<(C + 127) / 128, 128, 0, as_stream(stream)>>>(
+        nullptr, C, 1.0, gamma, beta, eps, 0.f, const_cast<float*>(running_mean), const_cast<float*>(running_var),
+        mean_rstd, scale_shift);
+    A2F_CHECK_LAUNCH("bn_finalize_kernel");
+    count_launch();
     return A2F_OK;
 }
 
@@ -242,20 +293,21 @@ int a2f_bn_train_bwd(const float* dy, const float* y_relu, const float* z, const
                     batches > 0,
                 "a2f_bn_train_bwd: bad arguments");
     A2F_REQUIRE(workspace_bytes >= (size_t)2 * C * sizeof(double), "a2f_bn_train_bwd: workspace too small (2*C doubles)");
-    cudaStream_t s = as_stream(stream);
-    double* sums = static_cast<double*>(workspace);
-    A2F_CHECK_CUDA(cudaMemsetAsync(sums, 0, (size_t)2 * C * sizeof(double), s));
-    const long long rows = batches * rows_per_batch;
-    long long gy = (rows + 63) / 64;
-    if (gy > 256) gy = 256;
-    bn_bwd_reduce_kernel<<<dim3((C + 31) / 32, (unsigned)gy), 256, 0, s>>>(dy, y_relu, z, mean_rstd, C, rows_per_batch, ld,
-                                                                            batch_stride, batches, sums);
-    A2F_CHECK_LAUNCH("bn_bwd_reduce_kernel");
-    bn_bwd_apply_kernel<<<ew_blocks(rows * C), 256, 0, s>>>(dy, y_relu, z, mean_rstd, gamma, sums, (double)rows, C,
-                                                             rows_per_batch, ld, batch_stride, batches, dz, dgamma, dbeta);
-    A2F_CHECK_LAUNCH("bn_bwd_apply_kernel");
-    count_launch(2);
-    return A2F_OK;
+    return bn_bwd_launch<false>(dy, y_relu, z, mean_rstd, gamma, C, rows_per_batch, ld, batch_stride, batches, dz, dgamma,
+                                dbeta, workspace, stream);
+}
+
+int a2f_bn_frozen_bwd(const float* dy, const float* y_relu, const float* z, const float* mean_rstd, const float* gamma, int C,
+                      long long rows_per_batch, long long ld, long long batch_stride, long long batches, float* dz,
+                      float* dgamma, float* dbeta, void* workspace, size_t workspace_bytes, void* stream) {
+    int rc = require_sm100();
+    if (rc != A2F_OK) return rc;
+    A2F_REQUIRE(dy && z && mean_rstd && gamma && dz && dgamma && dbeta && workspace && C > 0 && rows_per_batch > 0 &&
+                    batches > 0,
+                "a2f_bn_frozen_bwd: bad arguments");
+    A2F_REQUIRE(workspace_bytes >= (size_t)2 * C * sizeof(double), "a2f_bn_frozen_bwd: workspace too small (2*C doubles)");
+    return bn_bwd_launch<true>(dy, y_relu, z, mean_rstd, gamma, C, rows_per_batch, ld, batch_stride, batches, dz, dgamma,
+                               dbeta, workspace, stream);
 }
 
 }  // extern "C"

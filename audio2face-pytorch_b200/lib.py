@@ -213,6 +213,9 @@ _SIGNATURES = {
                                c_void_p]),
     "a2f_bn_train_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_ll, c_ll, c_ll, c_ll, c_void_p,
                                  c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "a2f_bn_frozen_stats": (c_int, [c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
+    "a2f_bn_frozen_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_ll, c_ll, c_ll, c_ll, c_void_p,
+                                  c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "a2f_mfcc_frames": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p]),
     "a2f_mfcc_mel_db": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "a2f_mfcc_dct_resize": (c_int, [c_void_p, c_void_p, c_float, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p,

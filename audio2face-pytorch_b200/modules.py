@@ -314,14 +314,16 @@ class Audio2Mesh(_A2FModule):
         tmpl = template.reshape(bs, -1).contiguous().float()
         grad = torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())
         if self.training:
-            # model.train(): BatchNorm uses batch statistics and updates its running stats (conv_training.py)
+            # model.train(): each BatchNorm in train() uses batch statistics and updates its running stats, one put in
+            # eval() uses its running stats and leaves them alone (conv_training.py)
             from . import conv_training
             if grad:
                 return conv_training.ConvModelTrainFn.run(self, "audio2mesh", x, one_hot, tmpl)
             return conv_training.a2m_forward_train(self, x, one_hot, tmpl)[0]
         if grad:
-            raise L.A2FError("Audio2Mesh: gradients with eval-mode (frozen) BatchNorm are not built; call .train() or "
-                             "run under torch.no_grad()")
+            raise L.A2FError("Audio2Mesh: gradients in eval() mode are not built; run under torch.no_grad(), or, to train "
+                             "with frozen BatchNorm statistics, call model.train() and then .eval() on the BatchNorm2d "
+                             "layers (ConvModelTrainer(freeze_bn=True) does this) -- the same arithmetic for this model")
         P = self._packed()
         S = L.SIMT_F32
         if self.precision == "bf16":
@@ -460,15 +462,17 @@ class Song2Face(_A2FModule):
         tmpl = template.reshape(bs, -1).contiguous().float()
         grad = torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())
         if self.training:
-            # model.train(): BatchNorm uses batch statistics and updates its running stats; true-fp32 convolutions and LSTMs
-            # whatever the precision, the vertex head follows it as for Audio2Mesh (conv_training.py)
+            # model.train(): each BatchNorm in train() uses batch statistics and updates its running stats, one put in
+            # eval() uses its running stats; true-fp32 convolutions and LSTMs whatever the precision, the vertex head
+            # follows it as for Audio2Mesh (conv_training.py)
             from . import conv_training
             if grad:
                 return conv_training.ConvModelTrainFn.run(self, "song2face", x, one_hot, tmpl)
             return conv_training.s2f_forward_train(self, x, one_hot, tmpl)[0]
         if grad:
-            raise L.A2FError("Song2Face: gradients with eval-mode (frozen) BatchNorm are not built; call .train() or "
-                             "run under torch.no_grad()")
+            raise L.A2FError("Song2Face: gradients in eval() mode are not built; run under torch.no_grad(), or, to train "
+                             "with frozen BatchNorm statistics, call model.train() and then .eval() on the BatchNorm2d "
+                             "layers (ConvModelTrainer(freeze_bn=True) does this) -- the same arithmetic for this model")
         P = self._packed()
         bf = self.precision == "bf16"
         cur = ops.a2m_assemble(x, one_hot)                                   # [B,64,33]; column 0 is an unused zero pad

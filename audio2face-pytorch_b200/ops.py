@@ -1111,6 +1111,19 @@ def bn_train_stats(v: View, gamma, beta, eps, momentum, running_mean, running_va
     return mr, ss
 
 
+def bn_frozen_stats(gamma, beta, eps, running_mean, running_var):
+    """Eval-mode BatchNorm inside a training step -> (mean_rstd [2C], scale_shift [2C]) from the running statistics,
+    which are only read."""
+    _dev(gamma, beta, running_mean, running_var)
+    C = gamma.numel()
+    mr = torch.empty(2 * C, dtype=torch.float32, device=gamma.device)
+    ss = torch.empty(2 * C, dtype=torch.float32, device=gamma.device)
+    L.check(L.load().a2f_bn_frozen_stats(gamma.data_ptr(), beta.data_ptr(), eps, running_mean.data_ptr(),
+                                         running_var.data_ptr(), C, mr.data_ptr(), ss.data_ptr(), _stream()),
+            "a2f_bn_frozen_stats")
+    return mr, ss
+
+
 def affine_act(src: View, dst: View, scale_shift: Optional[torch.Tensor], act: int) -> None:
     _dev(src.buf, dst.buf, scale_shift)
     sc = scale_shift.data_ptr() if scale_shift is not None else None
@@ -1119,15 +1132,26 @@ def affine_act(src: View, dst: View, scale_shift: Optional[torch.Tensor], act: i
                                     src.batches, _stream()), "a2f_affine_act")
 
 
-def bn_train_bwd(dy: View, y_relu: Optional[View], z: View, mean_rstd, gamma, dz: View, dgamma, dbeta) -> None:
+def _bn_bwd(fn: str, dy: View, y_relu: Optional[View], z: View, mean_rstd, gamma, dz: View, dgamma, dbeta) -> None:
     _dev(dy.buf, z.buf, dz.buf, mean_rstd, gamma, dgamma, dbeta)
     for o in (y_relu, z, dz):
         if o is not None and (o.ld, o.bs, o.rows, o.batches, o.C) != (dy.ld, dy.bs, dy.rows, dy.batches, dy.C):
-            raise L.A2FError("bn_train_bwd: all views must share one layout")
+            raise L.A2FError(f"{fn[4:]}: all views must share one layout")
     ws = torch.empty(2 * dy.C, dtype=torch.float64, device=dy.buf.device)
-    L.check(L.load().a2f_bn_train_bwd(dy.ptr, y_relu.ptr if y_relu is not None else None, z.ptr, mean_rstd.data_ptr(),
-                                      gamma.data_ptr(), dy.C, dy.rows, dy.ld, dy.bs, dy.batches, dz.ptr, dgamma.data_ptr(),
-                                      dbeta.data_ptr(), ws.data_ptr(), ws.numel() * 8, _stream()), "a2f_bn_train_bwd")
+    L.check(getattr(L.load(), fn)(dy.ptr, y_relu.ptr if y_relu is not None else None, z.ptr, mean_rstd.data_ptr(),
+                                  gamma.data_ptr(), dy.C, dy.rows, dy.ld, dy.bs, dy.batches, dz.ptr, dgamma.data_ptr(),
+                                  dbeta.data_ptr(), ws.data_ptr(), ws.numel() * 8, _stream()), fn)
+
+
+def bn_train_bwd(dy: View, y_relu: Optional[View], z: View, mean_rstd, gamma, dz: View, dgamma, dbeta) -> None:
+    """Backward of a batch-statistics BatchNorm (mean_rstd from bn_train_stats); dgamma / dbeta accumulate."""
+    _bn_bwd("a2f_bn_train_bwd", dy, y_relu, z, mean_rstd, gamma, dz, dgamma, dbeta)
+
+
+def bn_frozen_bwd(dy: View, y_relu: Optional[View], z: View, mean_rstd, gamma, dz: View, dgamma, dbeta) -> None:
+    """Backward of an eval-mode BatchNorm inside a training step: mean_rstd = [running_mean, 1/sqrt(running_var + eps)],
+    constants of the step, so dz = gamma*rstd*dy (masked by y_relu > 0); dgamma / dbeta accumulate."""
+    _bn_bwd("a2f_bn_frozen_bwd", dy, y_relu, z, mean_rstd, gamma, dz, dgamma, dbeta)
 
 
 # ---------------------------------------------------------------------------------------------------- MFCC extractor

@@ -409,14 +409,22 @@ class ConvModelTrainer:
 
     One process per GPU; parameters / gradients / Adam moments in flat fp32 buffers, one all-reduce of the whole
     gradient (2.2 M floats for Audio2Mesh) and the fused Adam kernel.  BatchNorm statistics stay per replica (the
-    reference has no SyncBN)."""
+    reference has no SyncBN).
+
+    freeze_bn=True puts every nn.BatchNorm2d in eval() after model.train(): the fine-tuning recipe that normalises with
+    the running statistics and keeps them unchanged (conv_training._bn_fwd).  Parameters with requires_grad False (e.g.
+    frozen BatchNorm affines) are not trained."""
 
     def __init__(self, model, feature_extractor=None, lr: float = 1e-4, weight_decay: Optional[float] = None,
-                 betas=(0.9, 0.999), eps: float = 1e-8, group=None):
+                 betas=(0.9, 0.999), eps: float = 1e-8, group=None, freeze_bn: bool = False):
         from . import modules
         if not next(model.parameters()).is_cuda:
             raise L.A2FError("ConvModelTrainer runs on CUDA (sm_100a) only; there is no CPU fallback")
         self.model, self.feature_extractor = model.train(), feature_extractor
+        if freeze_bn:
+            for mod in model.modules():
+                if isinstance(mod, torch.nn.BatchNorm2d):
+                    mod.eval()
         self.loss = modules.VocaLoss()
         self.lr = float(lr)
         self.weight_decay = float(lr / 10 if weight_decay is None else weight_decay)

@@ -502,7 +502,14 @@ int a2f_channel_affine(void* x, int dtype, const float* scale, const float* shif
  *      updated with `momentum` and the unbiased variance, as torch.nn.BatchNorm2d does.  workspace: 2*C doubles.
  *  a2f_affine_act: out = act(in*scale[c] + shift[c]) (scale/shift NULL = identity); in and out may alias.
  *  a2f_bn_train_bwd: dz = d/dz of y = gamma*(z-mean)*rstd + beta given dy (masked by y_relu > 0 when a ReLU followed,
- *      y_relu NULL otherwise); dgamma / dbeta accumulate.  workspace: 2*C doubles. */
+ *      y_relu NULL otherwise); dgamma / dbeta accumulate.  workspace: 2*C doubles.
+ *  An eval-mode ("frozen") BatchNorm inside a training step (model.train(), the layer in eval()) normalises with its
+ *  running statistics, leaves them unchanged, and its mean / rstd are constants of the step:
+ *  a2f_bn_frozen_stats: mean_rstd = {running_mean, 1/sqrt(running_var + eps)} and scale_shift as a2f_bn_train_stats
+ *      writes them; reads the running statistics only.
+ *  a2f_bn_frozen_bwd: dz = gamma*rstd*dy_eff (dy_eff = dy masked by y_relu > 0 as above), dgamma += sum dy_eff*xhat,
+ *      dbeta += sum dy_eff.  Same arguments as a2f_bn_train_bwd, mean_rstd from a2f_bn_frozen_stats.
+ *      workspace: 2*C doubles. */
 int a2f_voca_assemble(const float* x, const float* one_hot, int n_onehot, float* out, int B, void* stream);
 int a2f_bn_train_stats(const float* x, int C, long long rows_per_batch, long long ld, long long batch_stride,
                        long long batches, const float* gamma, const float* beta, float eps, float momentum,
@@ -514,6 +521,11 @@ int a2f_affine_act(const float* in, float* out, const float* scale, const float*
 int a2f_bn_train_bwd(const float* dy, const float* y_relu, const float* z, const float* mean_rstd, const float* gamma, int C,
                      long long rows_per_batch, long long ld, long long batch_stride, long long batches, float* dz,
                      float* dgamma, float* dbeta, void* workspace, size_t workspace_bytes, void* stream);
+int a2f_bn_frozen_stats(const float* gamma, const float* beta, float eps, const float* running_mean,
+                        const float* running_var, int C, float* mean_rstd, float* scale_shift, void* stream);
+int a2f_bn_frozen_bwd(const float* dy, const float* y_relu, const float* z, const float* mean_rstd, const float* gamma, int C,
+                      long long rows_per_batch, long long ld, long long batch_stride, long long batches, float* dz,
+                      float* dgamma, float* dbeta, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * Losses (ref:src/loss/loss.py:24-55; FaceFormerLoss :4-17 is the same with bs = T after dropping an odd last
