@@ -375,7 +375,9 @@ A2F_D void stv4(bf16* p, float4 v) {
 
 // One warp per row, rows strided over the grid; per-warp dgamma / dbeta / dbias partials live in registers and are
 // combined through shared memory once per CTA, then added atomically (<= 2*148 CTAs).
-template <typename TD, typename TX, typename TO, int NV>
+// PGRAD_ONLY: dgamma / dbeta alone (the input gradient is not wanted: nothing below the LayerNorm trains); the
+// per-element data-gradient arithmetic and the dx stores are left out.
+template <typename TD, typename TX, typename TO, int NV, bool PGRAD_ONLY = false>
 __global__ void __launch_bounds__(256) layernorm_bwd_kernel(const TD* __restrict__ dy, const TX* __restrict__ x,
                                                             const float* __restrict__ gamma, float eps,
                                                             TO* __restrict__ dx, float* __restrict__ dgamma,
@@ -412,10 +414,13 @@ __global__ void __launch_bounds__(256) layernorm_bwd_kernel(const TD* __restrict
             xv[j].x *= rstd; xv[j].y *= rstd; xv[j].z *= rstd; xv[j].w *= rstd;      // xhat
             ab[j].x += dv[j].x; ab[j].y += dv[j].y; ab[j].z += dv[j].z; ab[j].w += dv[j].w;
             ag[j].x += dv[j].x * xv[j].x; ag[j].y += dv[j].y * xv[j].y; ag[j].z += dv[j].z * xv[j].z; ag[j].w += dv[j].w * xv[j].w;
-            dv[j].x *= gm[j].x; dv[j].y *= gm[j].y; dv[j].z *= gm[j].z; dv[j].w *= gm[j].w;      // g
-            s1 += (dv[j].x + dv[j].y) + (dv[j].z + dv[j].w);
-            s2 += (dv[j].x * xv[j].x + dv[j].y * xv[j].y) + (dv[j].z * xv[j].z + dv[j].w * xv[j].w);
+            if constexpr (!PGRAD_ONLY) {
+                dv[j].x *= gm[j].x; dv[j].y *= gm[j].y; dv[j].z *= gm[j].z; dv[j].w *= gm[j].w;      // g
+                s1 += (dv[j].x + dv[j].y) + (dv[j].z + dv[j].w);
+                s2 += (dv[j].x * xv[j].x + dv[j].y * xv[j].y) + (dv[j].z * xv[j].z + dv[j].w * xv[j].w);
+            }
         }
+        if constexpr (PGRAD_ONLY) continue;
         s1 = warp_sum(s1) * (1.f / C);
         s2 = warp_sum(s2) * (1.f / C);
 #pragma unroll
@@ -445,14 +450,15 @@ __global__ void __launch_bounds__(256) layernorm_bwd_kernel(const TD* __restrict
     };
     reduce_out(ag, dgamma);
     reduce_out(ab, dbeta);
-    reduce_out(as, dbias);
+    if constexpr (!PGRAD_ONLY) reduce_out(as, dbias);
 }
 
 // ------------------------------------------------------------------------------------------------ interp + LN backward
 // Forward (w2v_frontend.cu interp_ln_kernel): v = l0*x[i0] + l1*x[i1]; y = LN(v)*gamma + beta.  One warp per frame:
 // recompute v and its statistics, LayerNorm backward, scatter l0*dv / l1*dv into the fp32 gradient of the conv-stack
-// output with atomics (each source row receives <= ~3 frames), accumulate dgamma / dbeta.
-template <typename TI, typename TD, int C>
+// output with atomics (each source row receives <= ~3 frames), accumulate dgamma / dbeta.  PGRAD_ONLY: dgamma / dbeta
+// alone (the conv stack below does not train): no data-gradient arithmetic, no scatter, no din buffer.
+template <typename TI, typename TD, int C, bool PGRAD_ONLY = false>
 __global__ void __launch_bounds__(256) interp_ln_bwd_kernel(const TI* __restrict__ in, const TD* __restrict__ dy,
                                                             const float* __restrict__ gamma, float eps,
                                                             float* __restrict__ din, float* __restrict__ dgamma,
@@ -498,10 +504,13 @@ __global__ void __launch_bounds__(256) interp_ln_bwd_kernel(const TI* __restrict
             const float d = ld_as_float(dy + (long long)f * C + cc);
             ab[j] += d;
             ag[j] += d * v[j];
-            g[j] = d * gamma[cc];
-            s1 += g[j];
-            s2 += g[j] * v[j];
+            if constexpr (!PGRAD_ONLY) {
+                g[j] = d * gamma[cc];
+                s1 += g[j];
+                s2 += g[j] * v[j];
+            }
         }
+        if constexpr (PGRAD_ONLY) continue;
         s1 = warp_sum(s1) * (1.f / C);
         s2 = warp_sum(s2) * (1.f / C);
         float* d0 = din + ((long long)b * S + i0) * C;
@@ -953,7 +962,8 @@ int a2f_layernorm_bwd(const void* dy, int dy_dtype, const void* x, int x_dtype, 
                       int dx_dtype, float* dgamma, float* dbeta, float* dbias, long long rows, int C, void* stream) {
     int rc = require_sm100();
     if (rc != A2F_OK) return rc;
-    A2F_REQUIRE(dy && x && gamma && dx && rows >= 0, "a2f_layernorm_bwd: bad arguments");
+    A2F_REQUIRE(dy && x && gamma && rows >= 0, "a2f_layernorm_bwd: bad arguments");
+    A2F_REQUIRE(dx || (!dbias && (dgamma || dbeta)), "a2f_layernorm_bwd: without dx, dbias must be NULL and dgamma or dbeta set");
     A2F_REQUIRE(C == 512 || C == 768, "a2f_layernorm_bwd: C must be 512 or 768");
     A2F_REQUIRE(dy_dtype == x_dtype && x_dtype == dx_dtype, "a2f_layernorm_bwd: dy, x and dx must share a dtype");
     if (rows == 0) return A2F_OK;
@@ -962,12 +972,14 @@ int a2f_layernorm_bwd(const void* dy, int dy_dtype, const void* x, int x_dtype, 
     cudaStream_t s = as_stream(stream);
     const int grid = (int)blocks;
 #define A2F_LNB(T, NV)                                                                                                  \
-    layernorm_bwd_kernel<T, T, T, NV><<<grid, 256, 0, s>>>((const T*)dy, (const T*)x, gamma, eps, (T*)dx, dgamma, dbeta, \
-                                                            dbias, rows)
+    if (dx) layernorm_bwd_kernel<T, T, T, NV><<<grid, 256, 0, s>>>((const T*)dy, (const T*)x, gamma, eps, (T*)dx, dgamma, \
+                                                                    dbeta, dbias, rows);                                 \
+    else layernorm_bwd_kernel<T, T, T, NV, true><<<grid, 256, 0, s>>>((const T*)dy, (const T*)x, gamma, eps, nullptr,   \
+                                                                      dgamma, dbeta, nullptr, rows)
     if (x_dtype == A2F_BF16) {
-        if (C == 512) A2F_LNB(bf16, 4); else A2F_LNB(bf16, 6);
+        if (C == 512) { A2F_LNB(bf16, 4); } else { A2F_LNB(bf16, 6); }
     } else {
-        if (C == 512) A2F_LNB(float, 4); else A2F_LNB(float, 6);
+        if (C == 512) { A2F_LNB(float, 4); } else { A2F_LNB(float, 6); }
     }
 #undef A2F_LNB
     A2F_CHECK_LAUNCH("layernorm_bwd_kernel");
@@ -979,18 +991,28 @@ int a2f_interp_ln_bwd(const void* in, int in_dtype, const void* dy, int dy_dtype
                       float* din, float* dgamma, float* dbeta, int B, int S, int T, int C, void* stream) {
     int rc = require_sm100();
     if (rc != A2F_OK) return rc;
-    A2F_REQUIRE(in && dy && gamma && din && dgamma && dbeta && B > 0 && S > 0 && T > 0, "a2f_interp_ln_bwd: bad arguments");
+    A2F_REQUIRE(in && dy && gamma && dgamma && dbeta && B > 0 && S > 0 && T > 0, "a2f_interp_ln_bwd: bad arguments");
     A2F_REQUIRE(C == 512, "a2f_interp_ln_bwd: C must be 512");
     A2F_REQUIRE(in_dtype == dy_dtype, "a2f_interp_ln_bwd: in and dy must share a dtype");
     long long blocks = ((long long)B * T + 7) / 8;
     if (blocks > 2LL * sm_count()) blocks = 2LL * sm_count();
     cudaStream_t s = as_stream(stream);
-    if (in_dtype == A2F_BF16)
-        interp_ln_bwd_kernel<bf16, bf16, 512><<<(int)blocks, 256, 0, s>>>((const bf16*)in, (const bf16*)dy, gamma, eps, din,
-                                                                          dgamma, dbeta, B, S, T);
-    else
-        interp_ln_bwd_kernel<float, float, 512><<<(int)blocks, 256, 0, s>>>((const float*)in, (const float*)dy, gamma, eps,
-                                                                            din, dgamma, dbeta, B, S, T);
+    if (in_dtype == A2F_BF16) {
+        if (din)
+            interp_ln_bwd_kernel<bf16, bf16, 512><<<(int)blocks, 256, 0, s>>>((const bf16*)in, (const bf16*)dy, gamma, eps,
+                                                                              din, dgamma, dbeta, B, S, T);
+        else
+            interp_ln_bwd_kernel<bf16, bf16, 512, true><<<(int)blocks, 256, 0, s>>>((const bf16*)in, (const bf16*)dy, gamma,
+                                                                                    eps, nullptr, dgamma, dbeta, B, S, T);
+    } else {
+        if (din)
+            interp_ln_bwd_kernel<float, float, 512><<<(int)blocks, 256, 0, s>>>((const float*)in, (const float*)dy, gamma,
+                                                                                eps, din, dgamma, dbeta, B, S, T);
+        else
+            interp_ln_bwd_kernel<float, float, 512, true><<<(int)blocks, 256, 0, s>>>((const float*)in, (const float*)dy,
+                                                                                      gamma, eps, nullptr, dgamma, dbeta,
+                                                                                      B, S, T);
+    }
     A2F_CHECK_LAUNCH("interp_ln_bwd_kernel");
     count_launch();
     return A2F_OK;

@@ -37,8 +37,10 @@ class _PackCache:
         if hit is not None and isinstance(hit[1], dict) and "_refresh" in hit[1] and len(hit[0]) == len(sig) and \
                 all(a[0] == b[0] and a[2] == b[2] for a, b in zip(hit[0], sig)):
             # same storage, new contents (an optimizer step): re-derive into the existing buffers -- a handful of
-            # launches (ops.PackPlan) instead of ~150 per step, and pointers stay valid for captured graphs
-            hit[1]["_refresh"]()
+            # launches (ops.PackPlan) instead of ~150 per step, and pointers stay valid for captured graphs.  Only the
+            # operands of the sources that changed are re-derived (frozen parameters keep their version counter).
+            changed = frozenset(b[0] for a, b in zip(hit[0], sig) if a[1] != b[1])
+            hit[1]["_refresh"](changed)
             self._store[key] = (sig, hit[1])
             return hit[1]
         val = build()
@@ -511,12 +513,35 @@ class _Box(nn.Module):
     """Plain namespace module: owns parameters / sub-modules under reference-compatible names, never called."""
 
 
+class _FeatureEncoderBox(_Box):
+    """`audio_encoder.feature_extractor`: the freezing API of HF's Wav2Vec2FeatureEncoder."""
+
+    def __init__(self):
+        super().__init__()
+        self._requires_grad = True
+
+    def _freeze_parameters(self):
+        for param in self.parameters():
+            param.requires_grad = False
+        self._requires_grad = False
+
+
+class _Wav2Vec2Box(_Box):
+    """`audio_encoder`: the freezing API of HF's Wav2Vec2Model (the reference's FaceFormer calls it in its constructor
+    when it fine-tunes)."""
+
+    def freeze_feature_encoder(self):
+        """Stop the gradient computation of the conv feature encoder (7 conv weights, GroupNorm gamma / beta); the
+        training backward then stops above it (training.grad_plan)."""
+        self.feature_extractor._freeze_parameters()
+
+
 def _w2v_param_tree() -> nn.Module:
     """Parameter container with the state_dict keys of the reference's Wav2Vec2Model subclass
     (ref:src/model/wav2vec.py:87; transformers Wav2Vec2Config() base architecture, SURVEY.md App. B.3)."""
-    enc = _Box()
+    enc = _Wav2Vec2Box()
     enc.masked_spec_embed = nn.Parameter(torch.empty(768).uniform_())
-    fe = _Box()
+    fe = _FeatureEncoderBox()
     layers = []
     for i, k in enumerate((10, 3, 3, 3, 3, 2, 2)):
         lay = _Box()
@@ -714,13 +739,25 @@ class Faceformer(_A2FModule):
             plan.finalize()
             P["_plan"] = plan
 
-            def refresh():
-                plan.run()
-                fold_ca()
-                ops.pack_posconv_weight(pz.original0.detach().reshape(-1), pz.original1.detach(), dt, out=P["pos_w"])
-                ops.pack_feedback(self.vertice_map.weight.detach(), self.vertice_map.bias.detach(),
-                                  self.vertice_map_r.weight.detach(), self.vertice_map_r.bias.detach(), out=(wc, bc))
-                ops.pack_decoder_fold(d.self_attn.in_proj_weight.detach(), wc, self.PPE.pe.detach(), self.period, fold_w, fold_pe)
+            ca_mod = d.multihead_attn
+            ca_srcs = (ca_mod.in_proj_weight, ca_mod.in_proj_bias, ca_mod.out_proj.weight, ca_mod.out_proj.bias,
+                       self.audio_feature_map.weight, self.audio_feature_map.bias)
+            fb_srcs = (self.vertice_map.weight, self.vertice_map.bias, self.vertice_map_r.weight, self.vertice_map_r.bias)
+
+            def refresh(changed=None):
+                # changed: data pointers of the sources modified since the last derivation (None = all)
+                hit = lambda *ts: changed is None or any(t.data_ptr() in changed for t in ts)     # noqa: E731
+                plan.run(changed)
+                if hit(*ca_srcs):
+                    fold_ca()
+                if hit(pz.original0, pz.original1):
+                    ops.pack_posconv_weight(pz.original0.detach().reshape(-1), pz.original1.detach(), dt, out=P["pos_w"])
+                if hit(*fb_srcs):
+                    ops.pack_feedback(self.vertice_map.weight.detach(), self.vertice_map.bias.detach(),
+                                      self.vertice_map_r.weight.detach(), self.vertice_map_r.bias.detach(), out=(wc, bc))
+                if hit(*fb_srcs, d.self_attn.in_proj_weight, self.PPE.pe):
+                    ops.pack_decoder_fold(d.self_attn.in_proj_weight.detach(), wc, self.PPE.pe.detach(), self.period, fold_w,
+                                          fold_pe)
 
             for p_ in (self.vertice_map.weight, self.vertice_map_r.weight, pz.original0, pz.original1):
                 if not p_.is_contiguous():

@@ -695,14 +695,18 @@ class PackPlan:
     The drop-in modules derive every packed GEMM operand (bf16 casts, W^T data-gradient operands, implicit-GEMM conv
     layouts, the fused QKV weight) from the fp32 master parameters.  Source and destination pointers are stable across
     optimizer steps (parameters are updated in place, destinations are owned by the plan's user), so the job table is
-    uploaded once and `run()` re-derives all operands after every step."""
+    uploaded once and `run()` re-derives all operands after every step.  `run(changed)` re-derives only the operands
+    whose source is in `changed` (data pointers), still in one launch: the job table of each such subset is built and
+    uploaded once, at its first use (with frozen parameters the subset is the same at every optimizer step)."""
 
     def __init__(self, device):
         self.device = device
         self.jobs = []
+        self.src_ptrs = []      # per job: data pointer of its source tensor
         self.keep = []          # tensors the jobs point into (kept alive with the plan)
         self.table = None
         self.total_tiles = 0
+        self._subsets = {}      # tuple of job indices -> (device table, n_jobs, total_tiles); kept for captured graphs
 
     def add(self, src: torch.Tensor, dst: torch.Tensor, R: int, Cc: int, ld_r: int, ld_c: int, ldo_r: int, ldo_c: int,
             src_off: int = 0, dst_off: int = 0) -> None:
@@ -720,6 +724,7 @@ class PackPlan:
         j.tile0 = self.total_tiles
         self.total_tiles += ((int(R) + 31) // 32) * ((int(Cc) + 31) // 32)
         self.jobs.append(j)
+        self.src_ptrs.append(src.data_ptr())
         self.keep += [src, dst]
 
     def cast(self, src: torch.Tensor, dst: torch.Tensor, dst_off: int = 0) -> None:
@@ -737,20 +742,35 @@ class PackPlan:
         ldo = int(ldo if ldo is not None else dst.stride(0))
         self.add(src, dst, R, Cc, ld_r, ld_c, 1, ldo, src_off=src_off, dst_off=dst_off)
 
+    def _upload(self, jobs) -> torch.Tensor:
+        raw = bytes((L.CopyJob * len(jobs))(*jobs))
+        return torch.frombuffer(bytearray(raw), dtype=torch.uint8).to(self.device)
+
     def finalize(self) -> "PackPlan":
         if not self.jobs:
             raise L.A2FError("empty PackPlan")
-        arr = (L.CopyJob * len(self.jobs))(*self.jobs)
-        raw = bytes(arr)
-        host = torch.frombuffer(bytearray(raw), dtype=torch.uint8)
-        self.table = host.to(self.device)
+        self.table = self._upload(self.jobs)
         return self
 
-    def run(self) -> None:
+    def run(self, changed=None) -> None:
         if self.table is None:
             self.finalize()
-        L.check(L.load().a2f_strided_copy_jobs(self.table.data_ptr(), len(self.jobs), self.total_tiles, _stream()),
-                "a2f_strided_copy_jobs")
+        table, n, tiles = self.table, len(self.jobs), self.total_tiles
+        if changed is not None:
+            sel = tuple(i for i, p in enumerate(self.src_ptrs) if p in changed)
+            if not sel:
+                return
+            if len(sel) < len(self.jobs):
+                if sel not in self._subsets:
+                    jobs, t0 = [], 0
+                    for i in sel:
+                        j = L.CopyJob.from_buffer_copy(self.jobs[i])
+                        j.tile0 = t0
+                        t0 += ((j.R + 31) // 32) * ((j.C + 31) // 32)
+                        jobs.append(j)
+                    self._subsets[sel] = (self._upload(jobs), len(jobs), t0)
+                table, n, tiles = self._subsets[sel]
+        L.check(L.load().a2f_strided_copy_jobs(table.data_ptr(), n, tiles, _stream()), "a2f_strided_copy_jobs")
 
 
 def colsum(x: torch.Tensor, out: torch.Tensor, rows: Optional[int] = None, cols: Optional[int] = None,
@@ -820,25 +840,31 @@ def spec_mask_bwd(dh: torch.Tensor, mask_u8: torch.Tensor, dembed: torch.Tensor)
     return dh
 
 
-def layernorm_bwd(dy: torch.Tensor, x: torch.Tensor, gamma: torch.Tensor, dgamma: torch.Tensor, dbeta: torch.Tensor,
-                  dbias: Optional[torch.Tensor] = None, eps: float = 1e-5) -> torch.Tensor:
+def layernorm_bwd(dy: torch.Tensor, x: torch.Tensor, gamma: torch.Tensor, dgamma: Optional[torch.Tensor],
+                  dbeta: Optional[torch.Tensor], dbias: Optional[torch.Tensor] = None, eps: float = 1e-5,
+                  want_dx: bool = True) -> Optional[torch.Tensor]:
+    """-> dx, or None with want_dx=False (parameter gradients only: no data-gradient arithmetic, no dx buffer).
+    dgamma / dbeta may be None (not accumulated); dbias needs dx."""
     _dev(dy, x, gamma, dgamma, dbeta, dbias)
+    if not want_dx and dbias is not None:
+        raise L.A2FError("layernorm_bwd: the bias column sum needs the input gradient")
     rows, Cc = x.shape
-    dx = torch.empty_like(x)
-    L.check(L.load().a2f_layernorm_bwd(dy.data_ptr(), _dt(dy), x.data_ptr(), _dt(x), gamma.data_ptr(), eps, dx.data_ptr(),
-                                       _dt(dx), dgamma.data_ptr(), dbeta.data_ptr(), L.ptr(dbias), rows, Cc, _stream()),
+    dx = torch.empty_like(x) if want_dx else None
+    L.check(L.load().a2f_layernorm_bwd(dy.data_ptr(), _dt(dy), x.data_ptr(), _dt(x), gamma.data_ptr(), eps, L.ptr(dx),
+                                       _dt(x), L.ptr(dgamma), L.ptr(dbeta), L.ptr(dbias), rows, Cc, _stream()),
             "a2f_layernorm_bwd")
     return dx
 
 
 def interp_ln_bwd(x: torch.Tensor, dy: torch.Tensor, gamma: torch.Tensor, dgamma: torch.Tensor, dbeta: torch.Tensor,
-                  eps: float = 1e-5) -> torch.Tensor:
-    """x [B,S,512] saved input, dy [B,T,512] -> fp32 gradient wrt x."""
+                  eps: float = 1e-5, want_dx: bool = True) -> Optional[torch.Tensor]:
+    """x [B,S,512] saved input, dy [B,T,512] -> fp32 gradient wrt x, or None with want_dx=False (dgamma / dbeta only:
+    no zero-filled [B,S,512] buffer, no scatter)."""
     _dev(x, dy, gamma, dgamma, dbeta)
     B, S, Cc = x.shape
     T = dy.shape[1]
-    din = torch.zeros((B, S, Cc), dtype=torch.float32, device=x.device)
-    L.check(L.load().a2f_interp_ln_bwd(x.data_ptr(), _dt(x), dy.data_ptr(), _dt(dy), gamma.data_ptr(), eps, din.data_ptr(),
+    din = torch.zeros((B, S, Cc), dtype=torch.float32, device=x.device) if want_dx else None
+    L.check(L.load().a2f_interp_ln_bwd(x.data_ptr(), _dt(x), dy.data_ptr(), _dt(dy), gamma.data_ptr(), eps, L.ptr(din),
                                        dgamma.data_ptr(), dbeta.data_ptr(), B, S, T, Cc, _stream()), "a2f_interp_ln_bwd")
     return din
 

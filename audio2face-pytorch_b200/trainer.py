@@ -187,6 +187,11 @@ class FaceformerTrainer:
     (every replica skips the same layers).  A layer skipped by LayerDrop gets no gradient, and like torch.optim.Adam
     for `grad is None`, its parameters, moments and step count stay untouched that step.
 
+    Frozen parameters (requires_grad False when the trainer is constructed, e.g. after
+    `model.audio_encoder.freeze_feature_encoder()`) are not trained: they stay out of the flat buffers (no gradient, no
+    Adam moments, `.grad` stays None), the backward stops at the lowest trainable op, and only the packed operands of
+    trainable parameters are re-derived after each update.  Changing the trainable set later raises at the next step.
+
     Batch semantics (extension; the reference is batch-1): loss = mean over the utterances of the per-utterance
     FaceFormerLoss; across ranks the gradient is the average of the per-rank gradients (DDP semantics)."""
 
@@ -207,6 +212,8 @@ class FaceformerTrainer:
         self.flat = FlatBuffers(model.named_parameters(), training.grad_stage_of, training.N_GRAD_STAGES,
                                 skip=training.no_grad_params(model), order_in_stage=training.grad_order_in_stage,
                                 wire=self.wire, buckets=default_buckets(training.N_GRAD_STAGES, n_buckets))
+        # the flat buffers hold the parameters that require grad now: freezing or unfreezing one later would leave them wrong
+        self._requires_grad = frozenset(n for n, p in model.named_parameters() if p.requires_grad)
         self.exp_avg = torch.zeros_like(self.flat.params)
         self.exp_avg_sq = torch.zeros_like(self.flat.params)
         self.steps = 0
@@ -236,6 +243,11 @@ class FaceformerTrainer:
         device tensor {loss, rec_loss, vel_loss} [3] of the local shard."""
         from . import ops, training
         m = self.model
+        now = frozenset(n for n, p in m.named_parameters() if p.requires_grad)
+        if now != self._requires_grad:
+            diff = sorted(now ^ self._requires_grad)
+            raise L.A2FError(f"FaceformerTrainer: the set of trainable parameters changed after construction ({len(diff)} "
+                             f"parameters, e.g. {diff[0]}); freeze before constructing the trainer, or build a new one")
         audio = audio.contiguous().float()
         B = audio.shape[0]
         one_hot = one_hot.reshape(B, -1).contiguous().float()

@@ -640,11 +640,13 @@ int a2f_dropout_mask(const a2f_dropout_args* args, long long n, unsigned char* m
  * one dtype, A2F_F32 or A2F_BF16; y may alias x or resid).  The backward of a site is the same call on the gradient. */
 int a2f_dropout_apply(const void* x, const void* resid, void* y, int dtype, long long n, const a2f_dropout_args* args,
                       void* stream);
-/* LayerNorm backward over the last dim (C = 512 or 768): x is the saved LayerNorm INPUT.  dgamma / dbeta accumulate;
- * dbias (optional) accumulates the column sums of dx = the bias gradient of the Linear that produced x. */
+/* LayerNorm backward over the last dim (C = 512 or 768): x is the saved LayerNorm INPUT.  dgamma / dbeta accumulate
+ * (either may be NULL); dbias (optional) accumulates the column sums of dx = the bias gradient of the Linear that
+ * produced x.  dx may be NULL (then dbias must be NULL): parameter gradients only, the input gradient is not computed. */
 int a2f_layernorm_bwd(const void* dy, int dy_dtype, const void* x, int x_dtype, const float* gamma, float eps, void* dx,
                       int dx_dtype, float* dgamma, float* dbeta, float* dbias, long long rows, int C, void* stream);
-/* backward of a2f_interp_ln: `in` [B,S,C] is the saved input, dy [B,T,C]; din [B,S,C] fp32 is ACCUMULATED into. */
+/* backward of a2f_interp_ln: `in` [B,S,C] is the saved input, dy [B,T,C]; din [B,S,C] fp32 is ACCUMULATED into.
+ * din may be NULL: dgamma / dbeta only, the input gradient is not computed. */
 int a2f_interp_ln_bwd(const void* in, int in_dtype, const void* dy, int dy_dtype, const float* gamma, float eps,
                       float* din, float* dgamma, float* dbeta, int B, int S, int T, int C, void* stream);
 /* backward of a2f_conv0_gn_gelu given da = dL/d(output) [B,L0,512]; gn_stats = the [B,512] (mean, rstd) float2 block
