@@ -20,7 +20,7 @@
 //
 // Two kernels live here: gemm_ln_kernel (one GEMM + LayerNorm: a2f_gemm_ln, used by the training forward, which also stores
 // the pre-LayerNorm sum) and enc_block_kernel further down (up to four GEMM phases of an encoder layer back to back in the
-// same cluster: a2f_encoder_block / a2f_ffn_ln, the inference path).  Both use ln_tile_epilogue for their LayerNorm tiles.
+// same cluster: a2f_encoder_block, the inference path).  Both use ln_tile_epilogue for their LayerNorm tiles.
 #include "a2f_common.cuh"
 #include "gemm_params.cuh"
 
@@ -983,20 +983,4 @@ extern "C" int a2f_encoder_block(const a2f_encoder_block_args* args, void* strea
     A2F_REQUIRE(args != nullptr, "a2f_encoder_block: NULL args");
     A2F_REQUIRE(args->M >= 0 && args->N > 0 && args->F > 0, "a2f_encoder_block: bad M/N/F");
     return a2f::enc_block_tc(*args, a2f::as_stream(stream));
-}
-
-extern "C" int a2f_ffn_ln(const void* X, long long ldx, const void* W1, long long ldw1, const float* bias1, const void* W2,
-                          long long ldw2, const float* bias2, const float* gamma, const float* beta, float eps, void* scratch,
-                          long long ldf, void* out, long long ldo, int M, int N, int F, void* stream) {
-    a2f_encoder_block_args g;
-    memset(&g, 0, sizeof(g));
-    g.M = M; g.N = N; g.F = F;
-    g.h1 = const_cast<void*>(X); g.ld_h1 = ldx;
-    g.w1 = W1; g.ld_w1 = ldw1; g.b1 = bias1;
-    g.f = scratch; g.ld_f = ldf;
-    g.w2 = W2; g.ld_w2 = ldw2; g.b2 = bias2;
-    g.ln2_g = gamma; g.ln2_b = beta;
-    g.h_out = out; g.ld_hout = ldo;
-    g.eps = eps;
-    return a2f_encoder_block(&g, stream);
 }

@@ -116,8 +116,6 @@ _SIGNATURES = {
     "a2f_gemm_ln": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_void_p, c_void_p, c_ll, c_void_p, c_void_p, c_float, c_void_p, c_ll,
                             c_void_p, c_ll, c_int, c_int, c_int, c_void_p]),
     "a2f_encoder_block": (c_int, [C.POINTER(EncoderBlockArgs), c_void_p]),
-    "a2f_ffn_ln": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_void_p, c_void_p, c_ll, c_void_p, c_void_p, c_void_p, c_float,
-                           c_void_p, c_ll, c_void_p, c_ll, c_int, c_int, c_int, c_void_p]),
     "a2f_posconv": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "a2f_pack_posconv_weight": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "a2f_pack_conv1d_weight": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),

@@ -621,19 +621,9 @@ class Faceformer(_A2FModule):
         # Philox key of the dropout masks and seed of the LayerDrop draws (include/a2f.h); None = drawn from torch's default
         # generator at first use; FaceformerTrainer gives every replica rank 0's seed.
         self.dropout_seed = None
-        # bf16 inference: run the encoder's 24 post-LayerNorms inside the GEMM epilogues (a2f_gemm_ln); False = the separate
-        # layernorm_kernel launches (A/B switch for profiles/)
-        self.fuse_layernorm = True
-        # ... and everything of a layer except the attention as ONE kernel (a2f_encoder_block); False = GEMM and a2f_gemm_ln
-        # launches (bit-identical results; A/B switch for profiles/)
-        self.fuse_ffn = True
-        self.fuse_block = "attn_ffn_qkv"
         # bf16 inference, 32 / 64 / 128 utterances: the vertex head runs concurrently with the decoder rollout on the SMs the
         # rollout leaves idle (ops.rollout_and_head_stream); False = rollout, then head
         self.stream_head = True
-        # inference front end: audio statistics and conv0 moments in one pass over the raw audio; False = a2f_audio_stats, then
-        # the moments of the normalised audio (two passes, one launch more)
-        self.raw_moments = True
         self.dataset = "vocaset"
         self.period = 60
         self.fps = 60
@@ -784,12 +774,10 @@ class Faceformer(_A2FModule):
         B, N = audio.shape
         dev = audio.device
         gn = ae.feature_extractor.conv_layers[0].layer_norm
-        if stats is None and self.raw_moments:
+        if stats is None:
             # processor statistics and conv0 moments from ONE pass over the raw audio (a2f_conv0_gn_gelu_auto)
-            x, stats = ops.conv0_gn_gelu_auto(audio, P["conv0_w"], gn.weight.detach(), gn.bias.detach(), dt)
+            x, _ = ops.conv0_gn_gelu_auto(audio, P["conv0_w"], gn.weight.detach(), gn.bias.detach(), dt)
         else:
-            if stats is None:
-                stats = ops.audio_stats(audio)
             x = ops.conv0_gn_gelu(audio, stats, P["conv0_w"], gn.weight.detach(), gn.bias.detach(), dt)   # [B,L0,512]
         L_in = x.shape[1]
         for i, k in enumerate((3, 3, 3, 3, 2, 2)):
@@ -810,50 +798,33 @@ class Faceformer(_A2FModule):
         ops.layernorm(pre, ae.encoder.layer_norm.weight.detach(), ae.encoder.layer_norm.bias.detach(), h)
         qkv = torch.empty((M, 2304), dtype=dt, device=dev)
         att = torch.empty((M, 768), dtype=dt, device=dev)
-        pre32 = torch.empty((M, 768), dtype=dt, device=dev)     # pre-LayerNorm sums (bf16 on the tensor-core path)
         ffn = torch.empty((M, 3072), dtype=dt, device=dev)
-        fuse = bf and self.fuse_layernorm
-        h1 = torch.empty((M, 768), dtype=dt, device=dev) if fuse else None
         layers = list(zip(ae.encoder.layers, P["layers"]))
-        if fuse and self.fuse_ffn:
-            # Everything of a layer that is local to a block of rows can run as ONE kernel (a2f_encoder_block; cluster of three
-            # CTA pairs per 256-row block): fuse_block selects the phases -- "ffn" (W1, GELU, W2, residual, LayerNorm),
-            # "attn_ffn" (+ attention out-projection and its LayerNorm in front), "attn_ffn_qkv" (+ the NEXT layer's q|k|v
-            # projection behind).  All variants give the same bits; DESIGN.md section 4 has the timings.
-            with_o = self.fuse_block in ("attn_ffn", "attn_ffn_qkv")
-            with_q = self.fuse_block in ("ffn_qkv", "attn_ffn_qkv")
+        if bf:
+            # everything of a layer but the attention is ONE kernel (a2f_encoder_block; cluster of three CTA pairs per 256-row
+            # block): attention out-projection and its LayerNorm, W1, GELU, W2, residual, LayerNorm, and the NEXT layer's
+            # q|k|v projection.  DESIGN.md section 4 has the timings.
+            h1 = torch.empty((M, 768), dtype=dt, device=dev)
             h2 = torch.empty((M, 768), dtype=dt, device=dev)
             for i, (blk, W) in enumerate(layers):
-                if i == 0 or not with_q:
+                if i == 0:      # the later layers' q|k|v come out of the block kernel of the layer before
                     ops.gemm(h, W["qkv_w"], qkv, bias=W["qkv_b"], backend=be)
                 ops.mha(qkv, att, B, T)
-                nxt = layers[i + 1][1] if (with_q and i + 1 < len(layers)) else None
                 kw = {}
-                if with_o:
-                    kw.update(att=att, wo=W["o_w"], bo=blk.attention.out_proj.bias.detach(), h_in=h,
-                              ln1_g=blk.layer_norm.weight.detach(), ln1_b=blk.layer_norm.bias.detach())
-                else:
-                    ops.gemm_ln(att, W["o_w"], blk.attention.out_proj.bias.detach(), h, blk.layer_norm.weight.detach(),
-                                blk.layer_norm.bias.detach(), h1)
-                if nxt is not None:
+                if i + 1 < len(layers):
+                    nxt = layers[i + 1][1]
                     kw.update(wq=nxt["qkv_w"], bq=nxt["qkv_b"], qkv=qkv)
                 ops.encoder_block(h1, W["f1_w"], blk.feed_forward.intermediate_dense.bias.detach(), W["f2_w"],
                                   blk.feed_forward.output_dense.bias.detach(), blk.final_layer_norm.weight.detach(),
-                                  blk.final_layer_norm.bias.detach(), ffn, h2, **kw)
+                                  blk.final_layer_norm.bias.detach(), ffn, h2, att=att, wo=W["o_w"],
+                                  bo=blk.attention.out_proj.bias.detach(), h_in=h, ln1_g=blk.layer_norm.weight.detach(),
+                                  ln1_b=blk.layer_norm.bias.detach(), **kw)
                 h, h2 = h2, h
             return h
+        pre32 = torch.empty((M, 768), dtype=dt, device=dev)     # pre-LayerNorm sums
         for blk, W in layers:
             ops.gemm(h, W["qkv_w"], qkv, bias=W["qkv_b"], backend=be)
             ops.mha(qkv, att, B, T)
-            if fuse:
-                # both post-LayerNorms run in the epilogue of the GEMM in front of them (a2f_gemm_ln: cluster of three CTA
-                # pairs per 256-row block, row statistics over DSMEM, pre-LN sum kept fp32 in tensor memory)
-                ops.gemm_ln(att, W["o_w"], blk.attention.out_proj.bias.detach(), h, blk.layer_norm.weight.detach(),
-                            blk.layer_norm.bias.detach(), h1)
-                ops.gemm(h1, W["f1_w"], ffn, bias=blk.feed_forward.intermediate_dense.bias.detach(), act=L.ACT_GELU, backend=be)
-                ops.gemm_ln(ffn, W["f2_w"], blk.feed_forward.output_dense.bias.detach(), h1, blk.final_layer_norm.weight.detach(),
-                            blk.final_layer_norm.bias.detach(), h)
-                continue
             ops.gemm(att, W["o_w"], pre32, bias=blk.attention.out_proj.bias.detach(), resid=h, backend=be)
             ops.layernorm(pre32, blk.layer_norm.weight.detach(), blk.layer_norm.bias.detach(), h)
             ops.gemm(h, W["f1_w"], ffn, bias=blk.feed_forward.intermediate_dense.bias.detach(), act=L.ACT_GELU, backend=be)

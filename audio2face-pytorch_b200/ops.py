@@ -167,12 +167,6 @@ def encoder_block(h1: torch.Tensor, w1: torch.Tensor, b1: Optional[torch.Tensor]
     return h_out
 
 
-def ffn_ln(x: torch.Tensor, w1: torch.Tensor, b1: Optional[torch.Tensor], w2: torch.Tensor, b2: Optional[torch.Tensor],
-           gamma: torch.Tensor, beta: torch.Tensor, scratch: torch.Tensor, out: torch.Tensor, eps: float = 1e-5) -> torch.Tensor:
-    """out = LayerNorm(x + gelu(x @ w1^T + b1) @ w2^T + b2) * gamma + beta: the feed-forward half of encoder_block."""
-    return encoder_block(x, w1, b1, w2, b2, gamma, beta, scratch, out, eps=eps)
-
-
 def gemm_ln(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], resid: torch.Tensor, gamma: torch.Tensor,
             beta: torch.Tensor, out: torch.Tensor, eps: float = 1e-5, pre_out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """out = LayerNorm(a @ w^T + bias + resid) * gamma + beta in one tcgen05 kernel (a2f_gemm_ln): bf16 [M,K] x [N,K],

@@ -233,7 +233,6 @@ class FaceformerTrainer:
         training.set_dropout_rank(model, dist.get_rank() if _world() > 1 else 0)
         self._skipped_stages = frozenset()      # stages of the layers LayerDrop skipped in the last forward
         self._stage_steps = None                # per-stage Adam step counts once LayerDrop has skipped a stage
-        self.fuse_loss = True          # bf16 path: vertex head + losses in one kernel (False = head, loss_fwd, loss_bwd, cast)
         self._dy = None
         self._ws_head = None
 
@@ -256,7 +255,7 @@ class FaceformerTrainer:
         self._skipped_stages = frozenset()
         hook = (lambda st: self.flat.all_reduce_stage(st, self.group)) if (self.overlap and _world() > 1) else None
         T = audio.shape[1] * self.fps // 16000
-        if self.fuse_loss and m.precision == "bf16" and T >= 2 and T % 2 == 0:
+        if m.precision == "bf16" and T >= 2 and T % 2 == 0:
             # tensor-core path, even clip length: the vertex head runs with the losses fused into its epilogue
             # (a2f_vertex_head_loss): gt is read once, dL/dy leaves as bf16 in the layout the backward GEMMs read, the
             # 60 KB/frame prediction is never written.  (Odd clips drop their last frame from the loss, ref loss.py:12-15,

@@ -426,7 +426,7 @@ def forward_train(model, audio: torch.Tensor, one_hot: torch.Tensor, tmpl: torch
               pc=pc if keep("posconv") else None, pre=pre if keep("enc_ln") else None)
     layers = []
     # the dropout sites of a layer run unfused: GEMM + a2f_dropout_apply (+ the separate LayerNorm)
-    fuse_ln = bf and getattr(model, "fuse_layernorm", True) and ph == 0
+    fuse_ln = bf and ph == 0
     for li, (blk, W) in enumerate(zip(ae.encoder.layers, P["layers"])):
         if drop and li in drop["skip"]:
             layers.append(None)                   # LayerDrop: the layer is the identity and launches nothing

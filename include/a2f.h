@@ -184,10 +184,6 @@ typedef struct a2f_encoder_block_args {
     float eps;
 } a2f_encoder_block_args;
 int a2f_encoder_block(const a2f_encoder_block_args* args, void* stream);
-/* The feed-forward half alone: out = LayerNorm(X + gelu(X W1^T + bias1) W2^T + bias2) * gamma + beta. */
-int a2f_ffn_ln(const void* X, long long ldx, const void* W1, long long ldw1, const float* bias1, const void* W2,
-               long long ldw2, const float* bias2, const float* gamma, const float* beta, float eps, void* scratch,
-               long long ldf, void* out, long long ldo, int M, int N, int F, void* stream);
 
 
 /* ------------------------------------------------------------------------------------------------------------

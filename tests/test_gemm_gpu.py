@@ -230,11 +230,12 @@ def test_gemm_ln_fused_epilogue(a2f_lib, dev, M, N, K):
 @pytest.mark.gpu
 @pytest.mark.parametrize("M,N,F", [(4800, 768, 3072), (257, 768, 3072), (1, 768, 3072), (9000, 768, 3072), (12000, 768, 3072),
                                    (700, 512, 1024), (300, 256, 1024), (300, 256, 256)])
-def test_ffn_ln_one_kernel_equals_two(a2f_lib, dev, M, N, F):
-    """a2f_ffn_ln (W1 + GELU + W2 + residual + LayerNorm in one kernel; the intermediate goes TMA store -> L2 -> TMA load
-    between CTAs of a cluster, ordered by cluster-scope mbarriers) must give the SAME bits as a2f_gemm(GELU) followed by
-    a2f_gemm_ln, and match torch fp32.  Shapes: the bench batch, ragged / single-row blocks, more row blocks than resident
-    clusters (the per-round barriers wrap their parity), 2- and 1-pair clusters, 1 to 4 phase-1 tiles per pair."""
+def test_ffn_one_kernel_equals_two(a2f_lib, dev, M, N, F):
+    """a2f_encoder_block with only its feed-forward phases (no att, no wq: W1 + GELU + W2 + residual + LayerNorm in one
+    kernel; the intermediate goes TMA store -> L2 -> TMA load between CTAs of a cluster, ordered by cluster-scope mbarriers)
+    must give the SAME bits as a2f_gemm(GELU) followed by a2f_gemm_ln, and match torch fp32.  Shapes: the bench batch,
+    ragged / single-row blocks, more row blocks than resident clusters (the per-round barriers wrap their parity), 2- and
+    1-pair clusters, 1 to 4 phase-1 tiles per pair."""
     from a2f_b200 import ops, lib as L
     g = torch.Generator().manual_seed(M + N + F)
     x = torch.randn(M, N, generator=g).bfloat16().to(dev)
@@ -249,7 +250,7 @@ def test_ffn_ln_one_kernel_equals_two(a2f_lib, dev, M, N, F):
     for rep in range(3):                                # repeated: a stale scratch from the previous run must not be read
         scratch = torch.full((M, F), float("nan"), dtype=torch.bfloat16, device=dev) if rep == 0 else scratch
         out = torch.empty((M, N), dtype=torch.bfloat16, device=dev)
-        ops.ffn_ln(x, w1, b1, w2, b2, gamma, beta, scratch, out)
+        ops.encoder_block(x, w1, b1, w2, b2, gamma, beta, scratch, out)
         torch.cuda.synchronize()
         assert torch.equal(scratch, f_ref), rep
         assert torch.equal(out, want), (rep, float((out.float() - want.float()).abs().max()))

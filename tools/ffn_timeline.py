@@ -1,6 +1,6 @@
 """In-kernel timeline of a2f_encoder_block at the bench shape (M=4800, d=768, ff=3072, all four phases): stamps of the
 leader CTAs, and launch-to-launch gaps of four back-to-back launches (globaltimer).
-    python tools/ffn_timeline.py [ffn]        ("ffn": only the feed-forward phases, as a2f_ffn_ln)
+    python tools/ffn_timeline.py [ffn]        ("ffn": only the feed-forward phases, no att / wq)
 Slots: 0 entry, 1 setup done (barriers, TMEM, cluster sync, griddepcontrol.wait), 2 first operands landed, 3 MMAs of phase 0
 issued, 4 MMAs of the last phase-1 tile issued, 5 MMAs of phase 2 issued, 6 MMAs of the last phase-3 tile issued, 7 h1
 published, 8..11 phase-1 tile t stored and published, 12 epilogue enters the second LayerNorm tile, 13 its stores issued,
@@ -29,7 +29,7 @@ h1, f, ho, q = (h_in.clone() if only_ffn else bf(M, N)), bf(M, F), bf(M, N), bf(
 
 def run():
     if only_ffn:
-        ops.ffn_ln(h1, w1, b1, w2, b2, g2, be2, f, ho)
+        ops.encoder_block(h1, w1, b1, w2, b2, g2, be2, f, ho)
     else:
         ops.encoder_block(h1, w1, b1, w2, b2, g2, be2, f, ho, att=att, wo=wo, bo=bo, h_in=h_in, ln1_g=g1, ln1_b=be1,
                           wq=wq, bq=bq, qkv=q)
